@@ -63,7 +63,14 @@ def parse_args():
     ap.add_argument("--e2e-steps", type=int, default=0, help="0 = steps")
     ap.add_argument("--out-paf", default="", help="strong: also write the PAF here")
     ap.add_argument("--no-checksum", action="store_true", help="strong: skip the extra (untimed) pass that computes the order-independent PAF digest")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="weak: after the timed steps, write the results of the last one as DIR/<name>.npy (see OutputDump)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.scaling != "weak"):
+        ap.error("--dump-outputs needs --impl b200 --scaling weak")
+    return args
 
 
 def config_sequences(name, nseq):
@@ -164,6 +171,76 @@ class ClockSampler:
         if sm:
             out.update(sm_mhz=statistics.median(sm), sm_max_mhz=max(mx), reasons=sorted(reasons), samples=len(sm))
         return out
+
+
+class OutputDump:
+    """What a caller of the timed path receives for each pair (aw_result, through aw_batch_fetch), collected from the fetch of
+    the last timed step and written as float64 / float32 .npy files, at most LIMIT bytes in all, so that two builds can be
+    compared output for output on the same inputs:
+
+      pair_index                 position of each dumped pair in the pair list of the step
+      <field>                    one aw_result field per file (FIELDS), one row per dumped pair
+      paf_sample_index           positions of the pairs whose PAF line is dumped
+      paf_sample_offsets         start of each of those lines in paf_sample_bytes (one more entry than lines)
+      paf_sample_bytes           the lines' bytes (float32 codes 0..255)
+
+    Every pair is dumped when there are at most MAX_ROWS, else a sample drawn with a fixed seed; the PAF text is dumped for a
+    fixed-seed sample of MAX_PAF_LINES of those pairs, as many as fit in the remaining bytes."""
+
+    FIELDS = ("query_idx", "target_idx", "query_start", "query_end", "target_start", "target_end", "is_reverse", "status", "score",
+              "num_matches", "alignment_length", "paf_len")
+    LIMIT = 64 << 20
+    MAX_ROWS = 1 << 18
+    MAX_PAF_LINES = 1024
+
+    def __init__(self, npairs):
+        import numpy as np
+
+        rng = np.random.default_rng(0)
+        rows = np.arange(npairs) if npairs <= self.MAX_ROWS else np.sort(rng.choice(npairs, self.MAX_ROWS, replace=False))
+        paf_rows = np.sort(rng.choice(rows, min(len(rows), self.MAX_PAF_LINES), replace=False))
+        self.rows, self.paf_rows = rows, paf_rows
+        self.take = np.zeros(npairs, dtype=bool)
+        self.take[rows] = True
+        self.take_paf = np.zeros(npairs, dtype=bool)
+        self.take_paf[paf_rows] = True
+        self.n, self.vals, self.paf = 0, [], []
+
+    def add(self, r):
+        """aw_result callback of Batch.fetch, called once per pair in pair order; returns 0 (do not cancel)"""
+        import ctypes as C
+
+        i = self.n
+        self.n += 1
+        if self.take[i]:
+            self.vals.append(tuple(getattr(r, f) for f in self.FIELDS))
+            if self.take_paf[i]:
+                self.paf.append(C.string_at(r.paf, r.paf_len) if r.paf_len else b"")
+        return 0
+
+    def write(self, out_dir):
+        import numpy as np
+
+        if self.n != len(self.take):
+            raise SystemExit(f"--dump-outputs: the fetch delivered {self.n} results for {len(self.take)} pairs")
+        vals = np.asarray(self.vals, dtype=np.float64).reshape(len(self.rows), len(self.FIELDS))
+        arrays = {"pair_index": self.rows.astype(np.float64)}
+        arrays.update((f, vals[:, j].copy()) for j, f in enumerate(self.FIELDS))
+        # bytes left for the PAF text (float32 codes) after the other arrays, the sample's index and offsets and the .npy headers
+        room = (self.LIMIT - sum(a.nbytes for a in arrays.values()) - 16 * (len(self.paf_rows) + 1) - (1 << 16)) // 4
+        lines, used = [], 0
+        for line in self.paf:
+            if used + len(line) > room:
+                break
+            lines.append(line)
+            used += len(line)
+        arrays["paf_sample_index"] = self.paf_rows[: len(lines)].astype(np.float64)
+        arrays["paf_sample_offsets"] = np.concatenate([[0], np.cumsum([len(x) for x in lines])]).astype(np.float64)
+        arrays["paf_sample_bytes"] = np.frombuffer(b"".join(lines), dtype=np.uint8).astype(np.float32)
+        assert sum(a.nbytes for a in arrays.values()) <= self.LIMIT
+        os.makedirs(out_dir, exist_ok=True)
+        for name, a in arrays.items():
+            np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def cpu_sample_pairs(cfg, pairs, cores):
@@ -306,11 +383,8 @@ def main():
     for _ in range(args.warmup):
         batch.launch(sh)
     torch.cuda.synchronize()
-    batch.fetch(collect=False)
-    st = batch.stats()
-    if st["failed_pairs"]:
-        raise SystemExit(f"{st['failed_pairs']} pairs failed on the GPU path")
-    retried = st["pairs_retried"]
+    if args.warmup:  # a batch that was never launched has nothing to fetch
+        batch.fetch(collect=False)
     launches_per_step = 2  # orientation kernel + alignment kernel (memsets are not kernels of ours)
 
     # ---- timed: device-resident ----
@@ -326,8 +400,14 @@ def main():
     barrier()
     ms = ev0.elapsed_time(ev1)
     clocks = sampler.stop()
-    batch.fetch(collect=False)
+    dump = OutputDump(len(pairs)) if args.dump_outputs else None
+    batch.fetch(collect=False, callback=dump.add if dump else None)
     st = batch.stats()
+    if st["failed_pairs"]:
+        raise SystemExit(f"{st['failed_pairs']} pairs failed on the GPU path")
+    retried = st["pairs_retried"]
+    if dump:
+        dump.write(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"))
 
     # ---- timed: end to end through the host-facing C-ABI call, host buffers ----
     e2e_steps = args.e2e_steps or args.steps
