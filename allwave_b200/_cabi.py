@@ -14,8 +14,9 @@ _SO = os.path.join(_PKG, "liballwave_cuda.so")
 AW_OK = 0
 AW_EINVAL, AW_ENODEVICE, AW_ECUDA, AW_ENOMEM, AW_EUNSUPPORTED, AW_EWORKSPACE, AW_ECALLBACK, AW_EALIGN = -1, -2, -3, -4, -5, -6, -7, -8
 AW_ORIENT_MASH, AW_ORIENT_WFA, AW_ORIENT_FORWARD = 0, 1, 2
-AW_FLAG_CIGAR_BYTES, AW_FLAG_ORDERED, AW_FLAG_NO_PAF, AW_FLAG_PAF_BLOCKS = 1, 2, 4, 8
+AW_FLAG_CIGAR_BYTES, AW_FLAG_ORDERED, AW_FLAG_NO_PAF, AW_FLAG_PAF_BLOCKS, AW_FLAG_SCORE_ONLY = 1, 2, 4, 8, 16
 AW_MEMORY_HIGH, AW_MEMORY_MEDIUM, AW_MEMORY_LOW, AW_MEMORY_ULTRALOW = 0, 1, 2, 3
+AW_SCOPE_SCORE, AW_SCOPE_ALIGNMENT = 0, 1
 
 EXPORTS = [
     "aw_abi_version", "aw_strerror", "aw_last_error", "aw_device_count", "aw_create", "aw_destroy", "aw_set_option",
@@ -359,6 +360,10 @@ class Aligner:
             check(lib().aw_aligner_new_affine2p(ctx._h, match, mismatch, gap_open1, gap_ext1, gap_open2, gap_ext2, memory_mode, C.byref(h)),
                   "aw_aligner_new_affine2p")
         self._h = h
+
+    def set_alignment_scope(self, scope):
+        """AW_SCOPE_SCORE: align() computes the score only and cigar() is empty; AW_SCOPE_ALIGNMENT (default): both"""
+        check(lib().aw_aligner_set_alignment_scope(self._h, scope), "aw_aligner_set_alignment_scope")
 
     def align(self, pattern: bytes, text: bytes):
         return lib().aw_aligner_align(self._h, pattern, len(pattern), text, len(text))

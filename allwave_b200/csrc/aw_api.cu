@@ -245,6 +245,7 @@ struct aw_aligner {
     aw_ctx* ctx = nullptr;  // private context on the parent's device
     aw_params params;
     int memory_mode = AW_MEMORY_ULTRALOW;
+    int scope = AW_SCOPE_ALIGNMENT;
     int32_t score = 0;
     std::vector<uint8_t> cigar;
 };
@@ -721,12 +722,22 @@ extern "C" void aw_batch_destroy(aw_ctx* c, aw_batch* b) {
     delete b;
 }
 
+// score-only results carry no CIGAR and no PAF text
+static int check_flags(uint32_t flags) {
+    if ((flags & AW_FLAG_SCORE_ONLY) && (flags & (AW_FLAG_CIGAR_BYTES | AW_FLAG_PAF_BLOCKS))) {
+        aw_set_error("AW_FLAG_SCORE_ONLY cannot be combined with AW_FLAG_CIGAR_BYTES or AW_FLAG_PAF_BLOCKS");
+        return AW_EINVAL;
+    }
+    return AW_OK;
+}
+
 // (re)initialises a batch object for a new pair list; device / pinned buffers of an earlier use are kept (grow-only)
 static int batch_init(aw_ctx* c, aw_batch* b, const aw_params* params, int orientation_mode, const aw_pair* pairs, uint64_t npairs, uint32_t flags) {
     int rc = pen_from_params(params, &b->pen);
     if (rc) return rc;
     if (orientation_mode == AW_ORIENT_WFA && (rc = pen_from_params(&c->orient_params, &b->pen_orient))) return rc;
     b->orient = orientation_mode;
+    if (flags & AW_FLAG_SCORE_ONLY) flags |= AW_FLAG_NO_PAF;
     b->flags = flags;
     b->npairs = npairs;
     b->launched = false;
@@ -748,7 +759,9 @@ static int batch_init(aw_ctx* c, aw_batch* b, const aw_params* params, int orien
     }
     size_t idlen_max = 0;
     for (auto& s : c->ids) idlen_max = std::max(idlen_max, s.size());
-    b->text_cap = (flags & AW_FLAG_NO_PAF) ? sum_len / 2 + 64 * npairs + 1024 : sum_len + (257 + 2 * idlen_max) * npairs + 1024;
+    b->text_cap = (flags & AW_FLAG_SCORE_ONLY) ? 16
+                  : (flags & AW_FLAG_NO_PAF)    ? sum_len / 2 + 64 * npairs + 1024
+                                                : sum_len + (257 + 2 * idlen_max) * npairs + 1024;
     b->bytes_cap = (flags & AW_FLAG_CIGAR_BYTES) ? sum_len + 16 : 16;
     const size_t np1 = (size_t)std::max<uint64_t>(1, npairs);
     if ((rc = b->d_pairs.ensure(sizeof(aw_pair) * np1)) || (rc = b->d_isrev.ensure(np1)) || (rc = b->d_out.ensure(sizeof(AwPairOut) * np1)) ||
@@ -812,6 +825,7 @@ extern "C" int aw_batch_create(aw_ctx* c, const aw_params* params, int orientati
     *out = nullptr;
     if (npairs > 0xfffffff0ull) return AW_EINVAL;
     if (orientation_mode != AW_ORIENT_MASH && orientation_mode != AW_ORIENT_FORWARD && orientation_mode != AW_ORIENT_WFA) return AW_EINVAL;
+    if (int rc = check_flags(flags)) return rc;
     AW_CUDA_CHECK(cudaSetDevice(c->device));
     aw_batch* b = new aw_batch();
     int rc = batch_init(c, b, params, orientation_mode, pairs, npairs, flags);
@@ -844,9 +858,9 @@ struct LaunchCfg {
     unsigned long long seq2_cap;
 };
 
-template <int NT, int BITS, bool TWO, class WS, int CL = 1>
+template <int NT, int BITS, bool TWO, class WS, int CL = 1, bool SCORE = false>
 cudaError_t launch_align(const awk::KParams& P, int grid, size_t smem, cudaStream_t st) {
-    auto kern = awk::aw_align_kernel<NT, BITS, TWO, WS, CL>;
+    auto kern = SCORE ? awk::aw_score_kernel<NT, BITS, TWO, WS, CL> : awk::aw_align_kernel<NT, BITS, TWO, WS, CL>;
     // static + dynamic shared memory together decide whether the opt-in is needed (the kernels carry up to 28 KB of static
     // shared memory); query the static part once per instantiation
     static size_t static_smem = ~(size_t)0;
@@ -902,15 +916,21 @@ cudaError_t dispatch_align(const awk::KParams& P, int nt, int bits, bool two, bo
     // SlotMeta rings: forward + reverse, plus one per warp for the warp-parallel leaves of the chunked kernels (aw_wfa.cuh RM_N)
     const int rm_n = (AW_LEAFPAR && nt >= 64 && bits == 2 && cluster == 1) ? 2 + nt / 32 : 2;
     size_t smem = sizeof(awk::SlotMeta) * rm_n * (scope + 1) + sizeof(int) * 10 * scope + sizeof(unsigned long long) * nt + sizeof(int) * (10 * scope + 4);
+    // AW_FLAG_SCORE_ONLY: the score-only twin of every kernel (the orientation passes clear the flag: they need X+I+D)
+    const bool score = (P.flags & AW_FLAG_SCORE_ONLY) != 0;
     if (cluster == AW_CLUSTER_SIZE && nt == AW_CLUSTER_NT && bits == 2 && !ws16) {
-        if (two) return launch_align<AW_CLUSTER_NT, 2, true, int, AW_CLUSTER_SIZE>(P, grid, smem, st);
+        if (two)
+            return score ? launch_align<AW_CLUSTER_NT, 2, true, int, AW_CLUSTER_SIZE, true>(P, grid, smem, st)
+                         : launch_align<AW_CLUSTER_NT, 2, true, int, AW_CLUSTER_SIZE>(P, grid, smem, st);
 #ifndef AW_FAST_BUILD
-        return launch_align<AW_CLUSTER_NT, 2, false, int, AW_CLUSTER_SIZE>(P, grid, smem, st);
+        return score ? launch_align<AW_CLUSTER_NT, 2, false, int, AW_CLUSTER_SIZE, true>(P, grid, smem, st)
+                     : launch_align<AW_CLUSTER_NT, 2, false, int, AW_CLUSTER_SIZE>(P, grid, smem, st);
 #endif
     }
     if (cluster != 1) return cudaErrorInvalidConfiguration;
-#define AW_CASE(NT_, BITS_, TWO_, WS_, W16_) \
-    if (nt == NT_ && bits == BITS_ && two == TWO_ && ws16 == W16_) return launch_align<NT_, BITS_, TWO_, WS_>(P, grid, smem, st);
+#define AW_CASE(NT_, BITS_, TWO_, WS_, W16_)                         \
+    if (nt == NT_ && bits == BITS_ && two == TWO_ && ws16 == W16_) \
+        return score ? launch_align<NT_, BITS_, TWO_, WS_, 1, true>(P, grid, smem, st) : launch_align<NT_, BITS_, TWO_, WS_>(P, grid, smem, st);
 #ifndef AW_FAST_BUILD  // dev builds (-DAW_FAST_BUILD) keep only the two-piece 2-bit int16 kernels
     AW_CASE(32, 2, true, int, false)
     AW_CASE(32, 2, false, int, false)
@@ -1397,7 +1417,16 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
         r.query_idx = b->h_pairs[i].query_idx;
         r.target_idx = b->h_pairs[i].target_idx;
         r.is_reverse = (uint8_t)(o->is_reverse == 1);
-        if (o->status == AW_OK) {
+        if (o->status == AW_OK && (b->flags & AW_FLAG_SCORE_ONLY)) {
+            // End2End covers both sequences; there are no op counts, CIGAR or text to derive anything else from
+            r.status = AW_OK;
+            r.score = o->score;
+            r.query_end = c->lens[r.query_idx];
+            r.target_end = c->lens[r.target_idx];
+            b->stats[6] += o->cells;
+            b->stats[7] += o->steps;
+            for (int q = 0; q < 6; ++q) b->cyc[q] += o->cyc[q];
+        } else if (o->status == AW_OK) {
             r.status = AW_OK;
             r.score = o->score;
             r.query_end = o->n_m + o->n_x + o->n_d;
@@ -1476,6 +1505,7 @@ extern "C" int aw_align_stream(aw_ctx* c, const aw_params* params, int orientati
                                aw_result_cb cb, aw_paf_block_cb block_cb, void* user) {
     if (!c || !params || !next) return AW_EINVAL;
     if (orientation_mode != AW_ORIENT_MASH && orientation_mode != AW_ORIENT_FORWARD && orientation_mode != AW_ORIENT_WFA) return AW_EINVAL;
+    if (int rc = check_flags(flags)) return rc;
     AW_CUDA_CHECK(cudaSetDevice(c->device));
     aw_batch* slot[2] = {new aw_batch(), new aw_batch()};
     bool busy[2] = {false, false};
@@ -1527,6 +1557,7 @@ struct ArraySource {
 extern "C" int aw_align_pairs(aw_ctx* c, const aw_params* params, int orientation_mode, const aw_pair* pairs, uint64_t npairs, uint32_t flags,
                               aw_result_cb cb, void* user) {
     if (!c || !params || (npairs && !pairs)) return AW_EINVAL;
+    if (int rc = check_flags(flags)) return rc;
     if (npairs == 0) {  // still validates the parameters like a real call
         AwPen pen;
         return pen_from_params(params, &pen);
@@ -1578,7 +1609,12 @@ extern "C" int aw_aligner_new_affine2p(aw_ctx* ctx, int32_t match_, int32_t mism
     p.has_gap2_open = p.has_gap2_extend = 1;
     return aligner_new(ctx, p, memory_mode, out);
 }
-extern "C" int aw_aligner_set_alignment_scope(aw_aligner* a, int scope) { return !a ? AW_EINVAL : (scope == AW_SCOPE_ALIGNMENT ? AW_OK : AW_EUNSUPPORTED); }
+extern "C" int aw_aligner_set_alignment_scope(aw_aligner* a, int scope) {
+    if (!a) return AW_EINVAL;
+    if (scope != AW_SCOPE_ALIGNMENT && scope != AW_SCOPE_SCORE) return AW_EUNSUPPORTED;
+    a->scope = scope;
+    return AW_OK;
+}
 extern "C" int aw_aligner_set_alignment_span(aw_aligner* a, int span) { return !a ? AW_EINVAL : (span == AW_SPAN_END2END ? AW_OK : AW_EUNSUPPORTED); }
 extern "C" int aw_aligner_set_heuristic(aw_aligner* a, int h) { return !a ? AW_EINVAL : (h == AW_HEURISTIC_NONE ? AW_OK : AW_EUNSUPPORTED); }
 extern "C" int aw_aligner_get_memory_mode(const aw_aligner* a) { return a ? a->memory_mode : AW_EINVAL; }
@@ -1598,7 +1634,8 @@ extern "C" int aw_aligner_align(aw_aligner* a, const uint8_t* pattern, int32_t p
     a->score = INT32_MAX;
     if (aw_load_sequences(a->ctx, 2, seqs, lens, ids) != AW_OK) return AW_ALIGN_OOM;
     aw_pair pr = {0, 1};
-    int rc = aw_align_pairs(a->ctx, &a->params, AW_ORIENT_FORWARD, &pr, 1, AW_FLAG_CIGAR_BYTES | AW_FLAG_NO_PAF, aligner_cb, a);
+    const uint32_t flags = a->scope == AW_SCOPE_SCORE ? AW_FLAG_SCORE_ONLY : AW_FLAG_CIGAR_BYTES | AW_FLAG_NO_PAF;
+    int rc = aw_align_pairs(a->ctx, &a->params, AW_ORIENT_FORWARD, &pr, 1, flags, aligner_cb, a);
     if (rc == AW_OK) return AW_ALIGN_COMPLETED;
     return rc == AW_ENOMEM ? AW_ALIGN_OOM : AW_ALIGN_UNDEFINED;
 }

@@ -1025,8 +1025,11 @@ __device__ __forceinline__ unsigned long long block_excl_scan(unsigned long long
 // of the biWFA recursion, where a cluster barrier per step would dominate) are left to CTA 0 alone, which also does every
 // backtrace and the CIGAR / PAF emission.  The wavefront rings stay in global memory (L2 / HBM): at Mb scale one ring row is
 // megabytes.
-template <int NT, int BITS, bool TWO, class WS, int CL = 1>
-__global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const KParams P) {
+// SCORE (aw_score_kernel): the optimal penalty of each pair only.  The top-level breakpoint's score is the pair's score, so
+// nothing below it runs; a top level that is a base case runs its wavefronts to the end cell and skips the backtrace.  No
+// CIGAR, no text and no bytes are produced.
+template <int NT, int BITS, bool TWO, class WS, int CL, bool SCORE>
+__device__ __forceinline__ void align_driver(const KParams& P) {
     static_assert(CL == 1 || (NT >= 64 && BITS == 2 && sizeof(WS) == 4), "cluster kernels exist for the int32 chunked path only");
     constexpr int NCOMP = TWO ? 5 : 3;
     const unsigned crank = (CL > 1) ? cluster_ctarank() : 0u;  // this CTA's rank in its cluster
@@ -1248,6 +1251,7 @@ __global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const 
         unsigned w_steps = 0, w_bps = 0, w_base = 0, w_maxbase = 0;
         if (tid == 0) s_nruns = 0;
         int sp_n = 0;
+        int sc_pen = 0;  // SCORE: the pair's wavefront penalty (under pen.x, pen.o1, ... -- shifted when match_score < 0)
         {
             // wavefront_bialign: short sequences go straight to the base case
             SubProblem top = {0, PLEN, 0, TLEN, AW_COMP_M, AW_COMP_M, (max(PLEN, TLEN) <= AW_BIALIGN_FALLBACK_MIN_LENGTH) ? 0 : INT_MAX};
@@ -1754,7 +1758,9 @@ __global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const 
                             rotate_red();
                         }
                         __syncwarp();  // the warp's history rows and metadata are visible to all of its lanes
-                        if (status == ST_OK) n_leaf = bt_run(lf.ce, score, lp, lt, k_end);
+                        if constexpr (!SCORE) {
+                            if (status == ST_OK) n_leaf = bt_run(lf.ce, score, lp, lt, k_end);
+                        }
                         lscore = score;
                     }
                     if (lane == 0) {
@@ -1788,6 +1794,12 @@ __global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const 
                 }
                 for (int i = tid; i < RM_N * 3 * NRED; i += NT) (&red[0][0][0])[i] = INT_MIN;  // the warps rotated their rows on their own
                 red_i = 0;
+                if constexpr (SCORE) {  // the one leaf is the top level (a pure gap leaves -1 here, see K8); it has no runs to append
+                    sc_pen = s_leaf_score[0];
+                    n_pending = 0;
+                    cta_sync<NT>();
+                    return;
+                }
                 const unsigned long long lpart = P.runs_cap / NW;
                 for (int q = 0; q < n_pending && status == ST_OK; ++q) {
                     // append leaf q's runs (stored back to front) to the pair's CIGAR, merging with the last run when the op continues
@@ -2324,6 +2336,10 @@ __global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const 
                     do_base = true;
                 } else {
                     ++w_bps;
+                    if constexpr (SCORE) {  // the top-level breakpoint's score is the pair's optimal score
+                        sc_pen = bp.score;
+                        break;
+                    }
                     const int bh = bp.off_f, bv = bp.off_f - bp.k_f;
                     if (bv < 0 || bv > plen || bh < 0 || bh > tlen || sp_n + 2 > MAX_STACK) {
                         status = ST_FAIL_WORKSPACE;
@@ -2483,6 +2499,11 @@ __global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const 
                 }
                 if (CL > 1 && !solo) cluster_sync_all();  // the whole history is in place (and see the note after phase 2)
                 if (status != ST_OK) AW_DFS_FAIL;
+                if constexpr (SCORE) {  // the score at which the end cell is reached is the pair's score: no backtrace
+                    sc_pen = score;
+                    w_maxbase = max(w_maxbase, (unsigned)score);
+                    break;
+                }
                 if (CL > 1 && crank != 0) continue;  // the backtrace and the CIGAR belong to CTA 0
                 w_maxbase = max(w_maxbase, (unsigned)score);
                 cta_sync<NT>();  // history + meta visible to warp 0
@@ -2522,6 +2543,33 @@ __global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const 
         // =========== K8: statistics, score, PAF text ===========
         cta_sync<NT>();
         if (CL > 1 && crank != 0) continue;  // CTA 0 owns the pair's CIGAR; the others go and wait for the next pair
+        if constexpr (SCORE) {
+            if (tid == 0) {
+                long long p = sc_pen;
+                if (PLEN == 0 || TLEN == 0) {  // one pure gap, or nothing
+                    const long long len = PLEN + TLEN;
+                    p = len ? pen.o1 + len * pen.e1 : 0;
+                    if (TWO && len) p = min(p, pen.o2 + len * pen.e2);
+                }
+                // with match_score M < 0 the wavefronts ran on the shifted penalties (aw_wfa2_compat.h): every column gives up
+                // M/2 per consumed character, so the user's penalty is exactly (P' + M (plen + tlen)) / 2
+                if (pen.smatch < 0) p = (p + (long long)pen.smatch * (PLEN + TLEN)) / 2;
+                AwPairOut o;
+                memset(&o, 0, sizeof(o));
+                o.status = (status == ST_OK) ? AW_OK : AW_EWORKSPACE;
+                o.score = (status == ST_OK) ? (int32_t)-p : INT_MAX;
+                o.is_reverse = is_rev;
+                o.cells = w_cells;
+                o.steps = w_steps;
+                o.n_breakpoints = w_bps;
+                o.n_base = w_base;
+                o.max_base_score = w_maxbase;
+                for (int i = 0; i < 6; ++i) o.cyc[i] = cyc[i];
+                P.out[pair_i] = o;
+            }
+            cta_sync<NT>();
+            continue;
+        }
         const unsigned nruns = (status == ST_OK) ? s_nruns : 0;
         if (tid < 8) s_acc[tid] = 0;
         cta_sync<NT>();
@@ -2676,6 +2724,15 @@ __global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const 
         cta_sync<NT>();
     }
     if constexpr (CL > 1) cluster_sync_all();  // no CTA may exit while another one can still read its shared memory
+}
+
+template <int NT, int BITS, bool TWO, class WS, int CL = 1>
+__global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_align_kernel(const KParams P) {
+    align_driver<NT, BITS, TWO, WS, CL, false>(P);
+}
+template <int NT, int BITS, bool TWO, class WS, int CL = 1>
+__global__ void __launch_bounds__(NT, AW_CTAS_PER_SM(NT)) aw_score_kernel(const KParams P) {
+    align_driver<NT, BITS, TWO, WS, CL, true>(P);
 }
 #undef AW_DFS_FAIL
 #undef AW_DFS_FAIL_CTA0

@@ -251,6 +251,42 @@ int64_t awh_test_cancel(aw_ctx* ctx, uint64_t n, const char* const* ids, const u
     return -1;
 }
 
+// for_each_with_callback with the given aw_align_pairs flags (e.g. AW_FLAG_SCORE_ONLY) over all ordered pairs of the loaded
+// sequences, default AlignmentParams, mash orientation.  Per result, 8 values in `rows` (room for `cap` results): query_idx,
+// target_idx, score, is_reverse, query_end, target_end, cigar string length, PAF length.  Returns the number of results, -1 on error.
+int64_t awh_test_for_each(aw_ctx* ctx, uint64_t n, const char* const* ids, const uint64_t* lens, uint32_t flags, int64_t* rows, uint64_t cap) {
+    std::vector<Sequence> S(n);
+    for (uint64_t i = 0; i < n; ++i) {
+        S[i].id = ids[i];
+        S[i].seq.resize(lens[i]);  // lengths only: the sequences are already loaded in ctx
+    }
+    try {
+        Context c(ctx, false);
+        AllPairIterator it(c, S, AlignmentParams(), true, true, SparsificationStrategy::none());
+        uint64_t k = 0;
+        it.for_each_with_callback(
+            [&](const AlignmentResult& a) {
+                if (k < cap) {
+                    int64_t* r = rows + 8 * k;
+                    r[0] = (int64_t)a.query_idx;
+                    r[1] = (int64_t)a.target_idx;
+                    r[2] = a.score;
+                    r[3] = a.is_reverse ? 1 : 0;
+                    r[4] = (int64_t)a.query_end;
+                    r[5] = (int64_t)a.target_end;
+                    r[6] = (int64_t)a.cigar.size();
+                    r[7] = (int64_t)a.paf.size();
+                }
+                ++k;
+            },
+            flags);
+        return (int64_t)k;
+    } catch (const std::exception& e) {
+        g_msg = e.what();
+        return -1;
+    }
+}
+
 // wfa::validate_cigar_alignment (src/wfa.rs:105-176): 0 = valid, else 1 with the reference's message in msg_out
 int awh_validate_cigar(const uint8_t* cigar, uint64_t n, uint64_t query_len, uint64_t reference_len, char* msg_out /*>=160*/) {
     const std::string m = wfa::validate_cigar_alignment(cigar, (size_t)n, (size_t)query_len, (size_t)reference_len);

@@ -40,6 +40,8 @@ def lib():
                                   C.c_int, C.c_uint64, C.c_char_p, C.c_int, C.POINTER(C.c_double)]
         L.awh_test_cancel.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_char_p), C.POINTER(C.c_uint64), C.c_uint64, C.c_uint64, C.c_char_p]
         L.awh_test_cancel.restype = C.c_int64
+        L.awh_test_for_each.argtypes = [C.c_void_p, C.c_uint64, C.POINTER(C.c_char_p), C.POINTER(C.c_uint64), C.c_uint32, C.POINTER(C.c_int64), C.c_uint64]
+        L.awh_test_for_each.restype = C.c_int64
         L.awh_validate_cigar.argtypes = [C.c_char_p, C.c_uint64, C.c_uint64, C.c_uint64, C.c_char_p]
         L.awh_align_sequences.argtypes = [C.c_void_p, C.c_char_p, C.c_uint64, C.c_char_p, C.c_uint64, C.POINTER(C.c_int32), C.c_int, C.POINTER(C.c_int32),
                                           C.POINTER(C.c_uint64), C.POINTER(C.c_void_p)]
@@ -148,6 +150,21 @@ def cancel_probe(ctx, ids, lens, fail_at, chunk_pairs=0):
     msg = C.create_string_buffer(128)
     seen = lib().awh_test_cancel(ctx._h, n, ia, la, fail_at, chunk_pairs, msg)
     return seen, msg.value.decode()
+
+
+def for_each_rows(ctx, ids, lens, flags=0):
+    """AllPairIterator::for_each_with_callback(cb, flags) over every ordered pair (default params, mash orientation): one dict per
+    result with the numeric fields and the lengths of its CIGAR string and PAF line"""
+    n = len(ids)
+    ia = (C.c_char_p * max(1, n))(*[i.encode() for i in ids])
+    la = (C.c_uint64 * max(1, n))(*lens)
+    cap = n * n
+    rows = (C.c_int64 * (8 * max(1, cap)))()
+    k = lib().awh_test_for_each(ctx._h, n, ia, la, flags, rows, cap)
+    if k < 0:
+        raise RuntimeError(lib().awh_last_message().decode())
+    keys = ["query_idx", "target_idx", "score", "is_reverse", "query_end", "target_end", "cg_len", "paf_len"]
+    return [dict(zip(keys, rows[8 * i: 8 * i + 8])) for i in range(min(k, cap))]
 
 
 def validate_cigar_alignment(cigar: bytes, query_len: int, reference_len: int):

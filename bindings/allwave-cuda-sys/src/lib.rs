@@ -26,6 +26,7 @@ pub const AW_FLAG_CIGAR_BYTES: u32 = 1;
 pub const AW_FLAG_ORDERED: u32 = 2;
 pub const AW_FLAG_NO_PAF: u32 = 4;
 pub const AW_FLAG_PAF_BLOCKS: u32 = 8;
+pub const AW_FLAG_SCORE_ONLY: u32 = 16;
 
 // aw_memory_mode / aw_alignment_scope / aw_alignment_span / aw_heuristic / aw_alignment_status (lib_wfa2 names)
 pub const AW_MEMORY_HIGH: c_int = 0;

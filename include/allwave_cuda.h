@@ -99,6 +99,13 @@ typedef struct aw_aligner aw_aligner;
 #define AW_FLAG_NO_PAF 4u       /* skip PAF text (stats + cg only)                           */
 #define AW_FLAG_PAF_BLOCKS 8u   /* aw_align_stream: every PAF line is followed by '\n' in the device text arena and whole
                                    batches are handed to the block callback (the CLI's writer, src/main.rs:347-367)   */
+#define AW_FLAG_SCORE_ONLY 16u  /* the optimal score of each pair only (WFA2's score scope), without CIGAR or PAF; implies
+                                   AW_FLAG_NO_PAF, and AW_EINVAL with AW_FLAG_CIGAR_BYTES or AW_FLAG_PAF_BLOCKS.  Per result:
+                                   status, score, is_reverse and the indices as usual; query_start = target_start = 0 and
+                                   query_end / target_end = the sequence lengths (End2End covers both); num_matches =
+                                   alignment_length = 0; cigar_bytes, cg and paf are NULL with length 0.  A failed pair is
+                                   AW_EALIGN with score INT32_MAX (no sentinel line).  aw_batch_stats [2..4] are 0.
+                                   The biWFA recursion stops at its top level, whose breakpoint score is the optimal score. */
 
 /* ---- library / device ---- */
 int aw_abi_version(void);
@@ -190,7 +197,8 @@ int aw_aligner_new_affine(aw_ctx* ctx, int32_t match_, int32_t mismatch, int32_t
                           int memory_mode, aw_aligner** out);
 int aw_aligner_new_affine2p(aw_ctx* ctx, int32_t match_, int32_t mismatch, int32_t gap_opening1, int32_t gap_extension1,
                             int32_t gap_opening2, int32_t gap_extension2, int memory_mode, aw_aligner** out);
-int aw_aligner_set_alignment_scope(aw_aligner* a, int scope);   /* only AW_SCOPE_ALIGNMENT */
+/* AW_SCOPE_SCORE: align() computes the score only (AW_FLAG_SCORE_ONLY), cigar() is empty; AW_SCOPE_ALIGNMENT (default): both */
+int aw_aligner_set_alignment_scope(aw_aligner* a, int scope);
 int aw_aligner_set_alignment_span(aw_aligner* a, int span);     /* only AW_SPAN_END2END    */
 int aw_aligner_set_heuristic(aw_aligner* a, int heuristic);     /* only AW_HEURISTIC_NONE  */
 int aw_aligner_get_memory_mode(const aw_aligner* a);
