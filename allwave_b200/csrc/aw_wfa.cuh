@@ -1234,7 +1234,10 @@ __device__ __forceinline__ void align_driver(const KParams& P) {
                 tw = s_seq + pwords + 4 + 2;
             }
         }
-        const int koff = (min(PLEN + 1, W / 2) + RALIGN - 1) & ~(RALIGN - 1);  // diagonal k lives at index k + koff
+        // diagonal k lives at index k + koff.  In-bounds diagonals span [-PLEN, TLEN]: the positive side never needs more than
+        // TLEN + 1, so a row wide enough for both sides gives the rest to the negative side (a query much longer than its target
+        // drifts far below diagonal -W/2); a narrower row is split evenly.
+        const int koff = (min(PLEN + 1, max(W / 2, W - TLEN - 1 - RALIGN)) + RALIGN - 1) & ~(RALIGN - 1);
         const int kmin_alloc = -koff, kmax_alloc = W - 1 - koff;
 
         int status = seq_fits ? ST_OK : ST_FAIL_WORKSPACE;
