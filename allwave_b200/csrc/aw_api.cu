@@ -212,6 +212,17 @@ struct aw_ctx {
     cudaStream_t stream2 = nullptr;  // kernel stream of workspace set 1 (set 0 runs on `stream`)
 };
 
+// Layout of a batch's control block (aw_batch::d_ctl, and the one of each retry rung), zeroed before every launch: the
+// arena cursors and work-list counters its alignment passes advance with atomics.  The --wfa-orientation passes run before
+// the main pass and into their own results: each strand has its own next-pair counter, and both share one pair of arena
+// cursors.  A next-pair counter is 32 bits wide, in the low word of its slot.
+struct BatchCtl {
+    unsigned long long text_cursor, bytes_cursor;  // main pass: bytes used in the PAF text and CIGAR byte arenas
+    unsigned long long next_pair;                  // main pass: next entry of the work list
+    unsigned long long orient_next_pair[2];        // orientation passes: next entry of the work list, per strand
+    unsigned long long orient_text_cursor, orient_bytes_cursor;
+};
+
 struct aw_batch {
     AwPen pen;
     int orient = AW_ORIENT_MASH;
@@ -221,7 +232,7 @@ struct aw_batch {
     DevBuf d_pairs, d_isrev, d_order, d_out, d_text, d_bytes, d_ctl;
     DevBuf d_text2, d_off;              // AW_FLAG_PAF_BLOCKS: the text arena again in pair order, and the per-pair offsets (n+1)
     DevBuf d_out_f, d_out_r, d_strand;  // --wfa-orientation passes: per-strand results and a constant 0.. / 1.. strand array
-    AwPen pen_orient;  // d_ctl: [0] text cursor, [1] bytes cursor, [2] next_pair
+    AwPen pen_orient;
     uint64_t text_cap = 0, bytes_cap = 0;
     bool has_order = false;
     uint64_t max_p = 0, max_t = 0;
@@ -699,23 +710,10 @@ static int pen_from_params(const aw_params* p, AwPen* pen) {
 extern "C" void aw_batch_destroy(aw_ctx* c, aw_batch* b) {
     if (!b) return;
     if (c) cudaSetDevice(c->device);
-    if (b->launched) {  // never park buffers a kernel still uses
+    if (b->launched) {  // never park buffers a kernel still uses (the buffers' destructors park them)
         if (b->ev_done) cudaEventSynchronize(b->ev_done);
         if (b->last_stream) cudaStreamSynchronize(b->last_stream);
     }
-    b->d_pairs.release();
-    b->d_isrev.release();
-    b->d_order.release();
-    b->d_out.release();
-    b->d_text.release();
-    b->d_bytes.release();
-    b->d_ctl.release();
-    b->d_out_f.release();
-    b->d_out_r.release();
-    b->d_strand.release();
-    b->h_out.release();
-    b->h_text.release();
-    b->h_bytes.release();
     if (b->ev0) cudaEventDestroy(b->ev0);
     if (b->ev1) cudaEventDestroy(b->ev1);
     if (b->ev_done) cudaEventDestroy(b->ev_done);
@@ -765,7 +763,7 @@ static int batch_init(aw_ctx* c, aw_batch* b, const aw_params* params, int orien
     b->bytes_cap = (flags & AW_FLAG_CIGAR_BYTES) ? sum_len + 16 : 16;
     const size_t np1 = (size_t)std::max<uint64_t>(1, npairs);
     if ((rc = b->d_pairs.ensure(sizeof(aw_pair) * np1)) || (rc = b->d_isrev.ensure(np1)) || (rc = b->d_out.ensure(sizeof(AwPairOut) * np1)) ||
-        (rc = b->d_text.ensure(b->text_cap)) || (rc = b->d_bytes.ensure(b->bytes_cap)) || (rc = b->d_ctl.ensure(64)) ||
+        (rc = b->d_text.ensure(b->text_cap)) || (rc = b->d_bytes.ensure(b->bytes_cap)) || (rc = b->d_ctl.ensure(sizeof(BatchCtl))) ||
         (orientation_mode == AW_ORIENT_WFA &&
          ((rc = b->d_out_f.ensure(sizeof(AwPairOut) * np1)) || (rc = b->d_out_r.ensure(sizeof(AwPairOut) * np1)) || (rc = b->d_strand.ensure(2 * np1)))))
         return rc;
@@ -1041,45 +1039,79 @@ int plan_launch(aw_ctx* c, const AwPen& pen, uint64_t npairs, uint64_t max_p, ui
     cfg->blk_cap = (int)(W / (awk::VBLOCK_CHUNKS * 4) + 2);  // blocks of >= 30 x 4 diagonals
     // pairs too long for the shared-memory staging keep their 4 word-pair arrays (pattern, text, both reversed) per CTA
     cfg->seq2_cap = (!ws16 && nt >= 64 && c->all_clean) ? 2 * ((max_p / 16 + 2) + (max_t / 16 + 2)) : 0;
-    int rc;
     // growing a workspace re-allocates it: a kernel of an earlier batch that is still running must not lose its buffers
-    if (grid * ws_ints * 4 > w.ws_main.cap || grid * 2ull * (pen.scope + 1) * (uint64_t)cfg->blk_cap * 2 * 4 > w.ws_blk.cap ||
-        grid * cfg->seq2_cap * 8 + 16 > w.ws_seq2.cap || grid * (uint64_t)hist_max_scores * awk::HIST_META_INTS * 4 > w.ws_hist_meta.cap ||
-        grid * runs_cap * 8 > w.ws_runs.cap)
-        if (cudaStreamSynchronize(kst) != cudaSuccess) return AW_ECUDA;
-    if ((rc = w.ws_main.ensure(grid * ws_ints * 4)) ||
-        (rc = w.ws_blk.ensure(grid * 2ull * (pen.scope + 1) * (uint64_t)cfg->blk_cap * 2 * 4)) ||
-        (rc = w.ws_seq2.ensure(grid * cfg->seq2_cap * 8 + 16)) ||
-        (rc = w.ws_hist_meta.ensure(grid * (uint64_t)hist_max_scores * awk::HIST_META_INTS * 4)) || (rc = w.ws_runs.ensure(grid * runs_cap * 8)))
-        return rc;
+    const std::pair<DevBuf*, uint64_t> need[] = {
+        {&w.ws_main, grid * ws_ints * 4},
+        {&w.ws_blk, grid * 2ull * (pen.scope + 1) * (uint64_t)cfg->blk_cap * 2 * 4},
+        {&w.ws_seq2, grid * cfg->seq2_cap * 8 + 16},
+        {&w.ws_hist_meta, grid * (uint64_t)hist_max_scores * awk::HIST_META_INTS * 4},
+        {&w.ws_runs, grid * runs_cap * 8},
+    };
+    for (const auto& n : need)
+        if (n.second > n.first->cap) {
+            if (cudaStreamSynchronize(kst) != cudaSuccess) return AW_ECUDA;
+            break;
+        }
+    for (const auto& n : need)
+        if (int rc = n.first->ensure(n.second)) return rc;
     return AW_OK;
 }
 
-void fill_params(aw_ctx* c, aw_batch* b, const AwPen& pen, const LaunchCfg& cfg, awk::KParams* P) {
-    memset(P, 0, sizeof(*P));
-    P->slots = c->d_slots.as<AwSlot>();
-    P->packed = c->d_packed.as<uint32_t>();
-    P->ascii = c->d_ascii.as<uint8_t>();
-    P->ids = c->d_ids.as<char>();
-    P->id_off = c->d_id_off.as<uint32_t>();
-    P->pairs = b->d_pairs.as<aw_pair>();
-    P->is_reverse = b->d_isrev.as<uint8_t>();
-    P->pen = pen;
-    P->flags = b->flags;
+// launches one alignment pass of batch b on the workspace set of the batch: the pairs order[0 .. npairs) (0 .. npairs
+// without an order) with the strands is_reverse, results into out, PAF text and CIGAR bytes into the two arenas
+cudaError_t launch_pass(aw_ctx* c, aw_batch* b, const AwPen& pen, const LaunchCfg& cfg, uint32_t flags, const uint8_t* is_reverse,
+                        const uint32_t* order, uint64_t npairs, AwPairOut* out, char* text, uint64_t text_cap, uint8_t* bytes, uint64_t bytes_cap,
+                        unsigned long long* text_cursor, unsigned long long* bytes_cursor, unsigned long long* next_pair, cudaStream_t st) {
+    awk::KParams P;
+    memset(&P, 0, sizeof(P));
+    P.slots = c->d_slots.as<AwSlot>();
+    P.packed = c->d_packed.as<uint32_t>();
+    P.ascii = c->d_ascii.as<uint8_t>();
+    P.ids = c->d_ids.as<char>();
+    P.id_off = c->d_id_off.as<uint32_t>();
+    P.pairs = b->d_pairs.as<aw_pair>();
+    P.is_reverse = is_reverse;
+    P.order = order;
+    P.npairs = (uint32_t)npairs;
+    P.next_pair = reinterpret_cast<unsigned int*>(next_pair);
+    P.pen = pen;
+    P.flags = flags;
     const aw_ctx::Workspace& w = c->wsp[b->slot];
-    P->ws = w.ws_main.as<int>();
-    P->ws_ints_per_cta = cfg.ws_ints;
-    P->W = cfg.W;
-    P->hist_ints = (int)std::min<unsigned long long>(cfg.hist_ints, 0x7fffffffull);
-    P->ws_hist_meta = w.ws_hist_meta.as<int>();
-    P->ws_blk = w.ws_blk.as<int>();
-    P->blk_cap = cfg.blk_cap;
-    P->ws_seq2 = w.ws_seq2.as<uint2>();
-    P->seq2_cap = cfg.seq2_cap;
-    P->hist_max_scores = cfg.hist_max_scores;
-    P->ws_runs = w.ws_runs.as<uint32_t>();
-    P->runs_cap = cfg.runs_cap;
-    P->solo_len = (int)std::min<int64_t>(c->solo_len, 0x7fffffff);
+    P.ws = w.ws_main.as<int>();
+    P.ws_ints_per_cta = cfg.ws_ints;
+    P.W = cfg.W;
+    P.hist_ints = (int)std::min<unsigned long long>(cfg.hist_ints, 0x7fffffffull);
+    P.ws_hist_meta = w.ws_hist_meta.as<int>();
+    P.ws_blk = w.ws_blk.as<int>();
+    P.blk_cap = cfg.blk_cap;
+    P.ws_seq2 = w.ws_seq2.as<uint2>();
+    P.seq2_cap = cfg.seq2_cap;
+    P.hist_max_scores = cfg.hist_max_scores;
+    P.ws_runs = w.ws_runs.as<uint32_t>();
+    P.runs_cap = cfg.runs_cap;
+    P.out = out;
+    P.text = text;
+    P.text_cursor = text_cursor;
+    P.text_cap = text_cap;
+    P.bytes = bytes;
+    P.bytes_cursor = bytes_cursor;
+    P.bytes_cap = bytes_cap;
+    P.solo_len = (int)std::min<int64_t>(c->solo_len, 0x7fffffff);
+    return dispatch_align(P, cfg.nt, c->all_clean ? 2 : 8, pen.two_piece != 0, cfg.ws16, cfg.grid, st, cfg.cluster);
+}
+
+// determine_orientation_wfa's two alignments: the pairs order[0 .. npairs) with the orientation penalties, forward and
+// reverse-complemented query, counts only (flags without AW_FLAG_SCORE_ONLY: the pick needs X+I+D), into d_out_f / d_out_r
+cudaError_t launch_orientation(aw_ctx* c, aw_batch* b, const LaunchCfg& cfo, const uint32_t* order, uint64_t npairs, BatchCtl* ctl, cudaStream_t st) {
+    const size_t np1 = (size_t)std::max<uint64_t>(1, b->npairs);
+    for (int s = 0; s < 2; ++s) {
+        cudaError_t e = launch_pass(c, b, b->pen_orient, cfo, AW_KFLAG_COUNT_ONLY | AW_FLAG_NO_PAF, b->d_strand.as<uint8_t>() + s * np1, order, npairs,
+                                    (s == 0 ? b->d_out_f : b->d_out_r).as<AwPairOut>(), b->d_text.as<char>(), b->text_cap, b->d_bytes.as<uint8_t>(),
+                                    b->bytes_cap, &ctl->orient_text_cursor, &ctl->orient_bytes_cursor, &ctl->orient_next_pair[s], st);
+        if (e != cudaSuccess) return e;
+        ++b->stats[0];
+    }
+    return cudaSuccess;
 }
 
 }  // namespace
@@ -1107,58 +1139,31 @@ extern "C" int aw_batch_launch(aw_ctx* c, aw_batch* b, void* stream) {
     }
     LaunchCfg cfg;
     if ((rc = plan_launch(c, b->pen, b->npairs, b->max_p, b->max_t, 0, &cfg, b->slot))) return rc;
-    AW_CUDA_CHECK(cudaMemsetAsync(b->d_ctl.p, 0, 64, st));
+    AW_CUDA_CHECK(cudaMemsetAsync(b->d_ctl.p, 0, sizeof(BatchCtl), st));
+    BatchCtl* ctl = b->d_ctl.as<BatchCtl>();
+    const uint32_t* order = b->has_order ? b->d_order.as<uint32_t>() : nullptr;
     if (b->orient == AW_ORIENT_WFA) {
         // determine_orientation_wfa: two full alignments with the orientation penalties, forward and
         // reverse-complemented query, statistics only; then pick the strand with fewer X+I+D columns
         LaunchCfg cfo;
         if ((rc = plan_launch(c, b->pen_orient, b->npairs, b->max_p, b->max_t, 0, &cfo, b->slot))) return rc;  // never larger than the main plan
-        const size_t np1 = (size_t)std::max<uint64_t>(1, b->npairs);
-        for (int strand = 0; strand < 2; ++strand) {
-            awk::KParams Q;
-            fill_params(c, b, b->pen_orient, cfo, &Q);
-            Q.flags = AW_KFLAG_COUNT_ONLY | AW_FLAG_NO_PAF;
-            Q.is_reverse = b->d_strand.as<uint8_t>() + strand * np1;
-            Q.order = b->has_order ? b->d_order.as<uint32_t>() : nullptr;
-            Q.npairs = (uint32_t)b->npairs;
-            Q.next_pair = reinterpret_cast<unsigned int*>(b->d_ctl.as<unsigned long long>() + 3 + strand);
-            Q.out = (strand == 0 ? b->d_out_f : b->d_out_r).as<AwPairOut>();
-            Q.text = b->d_text.as<char>();
-            Q.text_cursor = b->d_ctl.as<unsigned long long>() + 5;
-            Q.text_cap = b->text_cap;
-            Q.bytes = b->d_bytes.as<uint8_t>();
-            Q.bytes_cursor = b->d_ctl.as<unsigned long long>() + 6;
-            Q.bytes_cap = b->bytes_cap;
-            cudaError_t eo = dispatch_align(Q, cfo.nt, c->all_clean ? 2 : 8, b->pen_orient.two_piece != 0, cfo.ws16, cfo.grid, st, cfo.cluster);
-            if (eo != cudaSuccess) {
-                aw_set_error("orientation kernel launch: %s", cudaGetErrorString(eo));
-                return AW_ECUDA;
-            }
-            ++b->stats[0];
+        cudaError_t eo = launch_orientation(c, b, cfo, order, b->npairs, ctl, st);
+        if (eo != cudaSuccess) {
+            aw_set_error("orientation kernel launch: %s", cudaGetErrorString(eo));
+            return AW_ECUDA;
         }
         awk::aw_wfa_orient_pick_kernel<<<c->sm_count * 4, 256, 0, st>>>(b->d_out_f.as<AwPairOut>(), b->d_out_r.as<AwPairOut>(), b->npairs, b->d_isrev.as<uint8_t>());
         AW_CUDA_CHECK(cudaGetLastError());
         ++b->stats[0];
     }
-    awk::KParams P;
-    fill_params(c, b, b->pen, cfg, &P);
-    P.order = b->has_order ? b->d_order.as<uint32_t>() : nullptr;
-    P.npairs = (uint32_t)b->npairs;
-    P.next_pair = reinterpret_cast<unsigned int*>(b->d_ctl.as<unsigned long long>() + 2);
-    P.out = b->d_out.as<AwPairOut>();
-    P.text = b->d_text.as<char>();
-    P.text_cursor = b->d_ctl.as<unsigned long long>();
-    P.text_cap = b->text_cap;
-    P.bytes = b->d_bytes.as<uint8_t>();
-    P.bytes_cursor = b->d_ctl.as<unsigned long long>() + 1;
-    P.bytes_cap = b->bytes_cap;
     if (!b->ev0) {
         AW_CUDA_CHECK(cudaEventCreate(&b->ev0));
         AW_CUDA_CHECK(cudaEventCreate(&b->ev1));
         AW_CUDA_CHECK(cudaEventCreateWithFlags(&b->ev_done, cudaEventDisableTiming));
     }
     AW_CUDA_CHECK(cudaEventRecord(b->ev0, st));
-    cudaError_t e = dispatch_align(P, cfg.nt, c->all_clean ? 2 : 8, b->pen.two_piece != 0, cfg.ws16, cfg.grid, st, cfg.cluster);
+    cudaError_t e = launch_pass(c, b, b->pen, cfg, b->flags, b->d_isrev.as<uint8_t>(), order, b->npairs, b->d_out.as<AwPairOut>(), b->d_text.as<char>(),
+                                b->text_cap, b->d_bytes.as<uint8_t>(), b->bytes_cap, &ctl->text_cursor, &ctl->bytes_cursor, &ctl->next_pair, st);
     if (e != cudaSuccess) {
         aw_set_error("align kernel launch (nt=%d grid=%d): %s", cfg.nt, cfg.grid, cudaGetErrorString(e));
         return AW_ECUDA;
@@ -1176,58 +1181,62 @@ extern "C" int aw_batch_launch(aw_ctx* c, aw_batch* b, void* stream) {
     return AW_OK;
 }
 
+// One rung of a retry ladder: re-runs the pairs `todo` of batch b with the workspace plan_launch gives their longest query
+// and target at `attempt`.  launch(cfg, order, ctl, stream) queues the rung's passes over the uploaded work list `order`
+// with the zeroed control block `ctl` and returns an AW_ status.  The rung then waits for them and copies each result array
+// of `outs` back (all npairs entries), and the control block into *h_ctl when that is given.
+template <class Launch>
+static int retry_rung(aw_ctx* c, aw_batch* b, const AwPen& pen, const std::vector<uint32_t>& todo, int attempt, const char* what, Launch launch,
+                      std::initializer_list<std::pair<const DevBuf*, std::vector<AwPairOut>*>> outs, BatchCtl* h_ctl = nullptr) {
+    cudaStream_t kst = b->slot ? c->stream2 : c->stream;
+    uint64_t max_p = 0, max_t = 0;
+    for (uint32_t i : todo) {
+        max_p = std::max(max_p, c->lens[b->h_pairs[i].query_idx]);
+        max_t = std::max(max_t, c->lens[b->h_pairs[i].target_idx]);
+    }
+    LaunchCfg cfg;
+    int rc = plan_launch(c, pen, todo.size(), max_p, max_t, attempt, &cfg, b->slot);
+    if (rc) return rc;
+    DevBuf d_order, d_ctl;
+    if ((rc = d_order.ensure(4 * todo.size())) || (rc = d_ctl.ensure(sizeof(BatchCtl)))) return rc;
+    cudaError_t e = cudaMemcpy(d_order.p, todo.data(), 4 * todo.size(), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemset(d_ctl.p, 0, sizeof(BatchCtl));
+    if (e == cudaSuccess) {
+        if ((rc = launch(cfg, d_order.as<uint32_t>(), d_ctl.as<BatchCtl>(), kst))) return rc;
+        e = cudaStreamSynchronize(kst);
+    }
+    for (const auto& o : outs) {
+        o.second->resize(b->npairs);
+        if (e == cudaSuccess) e = cudaMemcpy(o.second->data(), o.first->p, sizeof(AwPairOut) * b->npairs, cudaMemcpyDeviceToHost);
+    }
+    if (e == cudaSuccess && h_ctl) e = cudaMemcpy(h_ctl, d_ctl.p, sizeof(BatchCtl), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) {
+        aw_set_error("%s: %s", what, cudaGetErrorString(e));
+        return AW_ECUDA;
+    }
+    return AW_OK;
+}
+
 // --wfa-orientation, pairs whose first-try orientation passes ran out of workspace (strand 2 = undecided): both count-only
 // passes go through the same ladder as the alignment itself, then the strand is picked like determine_orientation_wfa
 // (src/alignment.rs:157-175: a pass that still fails after the ladder counts as usize::MAX)
 static int retry_orientation(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
-    cudaStream_t kst = b->slot ? c->stream2 : c->stream;
     std::vector<uint32_t> todo;
     for (uint64_t i = 0; i < b->npairs; ++i)
         if (h_out[i].status == AW_EWORKSPACE && h_out[i].is_reverse > 1) todo.push_back((uint32_t)i);
     if (todo.empty()) return AW_OK;
-    const size_t np1 = (size_t)std::max<uint64_t>(1, b->npairs);
-    std::vector<AwPairOut> of(b->npairs), orv(b->npairs);
+    std::vector<AwPairOut> of, orv;
     std::vector<uint8_t> strand(b->npairs, 0);
     std::vector<uint8_t> have_f(b->npairs, 0), have_r(b->npairs, 0);
     std::vector<unsigned long long> ed_f(b->npairs, ~0ull), ed_r(b->npairs, ~0ull);
+    // at least one rung, also with max_retry_attempts = 0 (where retry_failed runs none)
     for (int attempt = 1; attempt <= std::max(1, c->max_retry) && !todo.empty(); ++attempt) {
-        uint64_t max_p = 0, max_t = 0;
-        for (uint32_t i : todo) {
-            max_p = std::max(max_p, c->lens[b->h_pairs[i].query_idx]);
-            max_t = std::max(max_t, c->lens[b->h_pairs[i].target_idx]);
-        }
-        LaunchCfg cfo;
-        int rc = plan_launch(c, b->pen_orient, todo.size(), max_p, max_t, attempt, &cfo, b->slot);
-        if (rc) return rc;
-        DevBuf d_order, d_ctl;
-        if ((rc = d_order.ensure(4 * todo.size())) || (rc = d_ctl.ensure(64))) return rc;
-        cudaError_t e = cudaMemcpy(d_order.p, todo.data(), 4 * todo.size(), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMemset(d_ctl.p, 0, 64);
-        for (int s = 0; s < 2 && e == cudaSuccess; ++s) {
-            awk::KParams Q;
-            fill_params(c, b, b->pen_orient, cfo, &Q);
-            Q.flags = AW_KFLAG_COUNT_ONLY | AW_FLAG_NO_PAF;
-            Q.is_reverse = b->d_strand.as<uint8_t>() + s * np1;
-            Q.order = d_order.as<uint32_t>();
-            Q.npairs = (uint32_t)todo.size();
-            Q.next_pair = reinterpret_cast<unsigned int*>(d_ctl.as<unsigned long long>() + 3 + s);
-            Q.out = (s == 0 ? b->d_out_f : b->d_out_r).as<AwPairOut>();
-            Q.text = b->d_text.as<char>();
-            Q.text_cursor = d_ctl.as<unsigned long long>() + 5;
-            Q.text_cap = b->text_cap;
-            Q.bytes = b->d_bytes.as<uint8_t>();
-            Q.bytes_cursor = d_ctl.as<unsigned long long>() + 6;
-            Q.bytes_cap = b->bytes_cap;
-            e = dispatch_align(Q, cfo.nt, c->all_clean ? 2 : 8, b->pen_orient.two_piece != 0, cfo.ws16, cfo.grid, kst, cfo.cluster);
-            ++b->stats[0];
-        }
-        if (e == cudaSuccess) e = cudaStreamSynchronize(kst);
-        if (e == cudaSuccess) e = cudaMemcpy(of.data(), b->d_out_f.p, sizeof(AwPairOut) * b->npairs, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(orv.data(), b->d_out_r.p, sizeof(AwPairOut) * b->npairs, cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) {
-            aw_set_error("orientation retry: %s", cudaGetErrorString(e));
-            return AW_ECUDA;
-        }
+        auto launch = [&](const LaunchCfg& cfo, const uint32_t* order, BatchCtl* ctl, cudaStream_t kst) -> int {
+            const cudaError_t e = launch_orientation(c, b, cfo, order, todo.size(), ctl, kst);
+            if (e != cudaSuccess) aw_set_error("orientation retry: %s", cudaGetErrorString(e));
+            return e == cudaSuccess ? AW_OK : AW_ECUDA;
+        };
+        if (int rc = retry_rung(c, b, b->pen_orient, todo, attempt, "orientation retry", launch, {{&b->d_out_f, &of}, {&b->d_out_r, &orv}})) return rc;
         std::vector<uint32_t> still;
         const bool last = attempt >= std::max(1, c->max_retry);
         for (uint32_t i : todo) {
@@ -1265,8 +1274,7 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
     b->stats[1] = failed.size();
     // a later batch may already be queued on this batch's kernel stream with the current workspace: let it finish before the
     // workspace is re-planned (and possibly re-allocated) for the retry
-    cudaStream_t kst = b->slot ? c->stream2 : c->stream;
-    AW_CUDA_CHECK(cudaStreamSynchronize(kst));
+    AW_CUDA_CHECK(cudaStreamSynchronize(b->slot ? c->stream2 : c->stream));
     if (b->orient == AW_ORIENT_WFA) {
         int rc = retry_orientation(c, b, h_out);
         if (rc) return rc;
@@ -1284,53 +1292,32 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
             failed.clear();
             break;
         }
-        uint64_t max_p = 0, max_t = 0, sum_len = 0;
+        uint64_t sum_len = 0;
         size_t idlen_max = 0;
         for (uint32_t i : failed) {
-            const uint64_t pl = c->lens[b->h_pairs[i].query_idx], tl = c->lens[b->h_pairs[i].target_idx];
-            max_p = std::max(max_p, pl);
-            max_t = std::max(max_t, tl);
-            sum_len += pl + tl;
+            sum_len += c->lens[b->h_pairs[i].query_idx] + c->lens[b->h_pairs[i].target_idx];
             idlen_max = std::max(idlen_max, c->ids[b->h_pairs[i].query_idx].size() + c->ids[b->h_pairs[i].target_idx].size());
         }
-        LaunchCfg cfg;
-        int rc = plan_launch(c, b->pen, failed.size(), max_p, max_t, attempt, &cfg, b->slot);
-        if (rc) return rc;
         const uint64_t text_cap = 12 * sum_len + (256 + idlen_max) * failed.size() + 1024;
         const uint64_t bytes_cap = (b->flags & AW_FLAG_CIGAR_BYTES) ? sum_len + 16 : 16;
-        DevBuf d_order, d_out, d_text, d_bytes, d_ctl;
-        if ((rc = d_order.ensure(4 * failed.size())) || (rc = d_out.ensure(sizeof(AwPairOut) * b->npairs)) || (rc = d_text.ensure(text_cap)) ||
-            (rc = d_bytes.ensure(bytes_cap)) || (rc = d_ctl.ensure(64)))
-            return rc;
-        cudaError_t e = cudaMemcpy(d_order.p, failed.data(), 4 * failed.size(), cudaMemcpyHostToDevice);
-        if (e == cudaSuccess) e = cudaMemset(d_ctl.p, 0, 64);
-        awk::KParams P;
-        fill_params(c, b, b->pen, cfg, &P);
-        P.order = d_order.as<uint32_t>();
-        P.npairs = (uint32_t)failed.size();
-        P.next_pair = reinterpret_cast<unsigned int*>(d_ctl.as<unsigned long long>() + 2);
-        P.out = d_out.as<AwPairOut>();
-        P.text = d_text.as<char>();
-        P.text_cursor = d_ctl.as<unsigned long long>();
-        P.text_cap = text_cap;
-        P.bytes = d_bytes.as<uint8_t>();
-        P.bytes_cursor = d_ctl.as<unsigned long long>() + 1;
-        P.bytes_cap = bytes_cap;
-        if (e == cudaSuccess) e = dispatch_align(P, cfg.nt, c->all_clean ? 2 : 8, b->pen.two_piece != 0, cfg.ws16, cfg.grid, kst, cfg.cluster);
-        ++b->stats[0];
-        if (e == cudaSuccess) e = cudaStreamSynchronize(kst);
-        std::vector<AwPairOut> outs(b->npairs);
-        unsigned long long ctl[3] = {0, 0, 0};
-        if (e == cudaSuccess) e = cudaMemcpy(outs.data(), d_out.p, sizeof(AwPairOut) * b->npairs, cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess) e = cudaMemcpy(ctl, d_ctl.p, 24, cudaMemcpyDeviceToHost);
-        std::vector<char> text(std::min<uint64_t>(ctl[0], text_cap));
-        std::vector<uint8_t> bytes(std::min<uint64_t>(ctl[1], bytes_cap));
-        if (e == cudaSuccess && !text.empty()) e = cudaMemcpy(text.data(), d_text.p, text.size(), cudaMemcpyDeviceToHost);
-        if (e == cudaSuccess && !bytes.empty()) e = cudaMemcpy(bytes.data(), d_bytes.p, bytes.size(), cudaMemcpyDeviceToHost);
-        if (e != cudaSuccess) {
-            aw_set_error("retry launch: %s", cudaGetErrorString(e));
-            return AW_ECUDA;
-        }
+        DevBuf d_out, d_text, d_bytes;
+        auto launch = [&](const LaunchCfg& cfg, const uint32_t* order, BatchCtl* ctl, cudaStream_t kst) -> int {
+            int rc;
+            if ((rc = d_out.ensure(sizeof(AwPairOut) * b->npairs)) || (rc = d_text.ensure(text_cap)) || (rc = d_bytes.ensure(bytes_cap))) return rc;
+            const cudaError_t e = launch_pass(c, b, b->pen, cfg, b->flags, b->d_isrev.as<uint8_t>(), order, failed.size(), d_out.as<AwPairOut>(),
+                                              d_text.as<char>(), text_cap, d_bytes.as<uint8_t>(), bytes_cap, &ctl->text_cursor, &ctl->bytes_cursor,
+                                              &ctl->next_pair, kst);
+            ++b->stats[0];
+            if (e != cudaSuccess) aw_set_error("retry launch: %s", cudaGetErrorString(e));
+            return e == cudaSuccess ? AW_OK : AW_ECUDA;
+        };
+        std::vector<AwPairOut> outs;
+        BatchCtl ctl;
+        if (int rc = retry_rung(c, b, b->pen, failed, attempt, "retry launch", launch, {{&d_out, &outs}}, &ctl)) return rc;
+        std::vector<char> text(std::min<uint64_t>(ctl.text_cursor, text_cap));
+        std::vector<uint8_t> bytes(std::min<uint64_t>(ctl.bytes_cursor, bytes_cap));
+        if (!text.empty()) AW_CUDA_CHECK(cudaMemcpy(text.data(), d_text.p, text.size(), cudaMemcpyDeviceToHost));
+        if (!bytes.empty()) AW_CUDA_CHECK(cudaMemcpy(bytes.data(), d_bytes.p, bytes.size(), cudaMemcpyDeviceToHost));
         std::vector<uint32_t> still;
         for (uint32_t i : failed) {
             AwPairOut o = outs[i];
@@ -1354,6 +1341,19 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
     return AW_OK;
 }
 
+// adds a pair's work counters to the batch's stats: CIGAR runs and alignment columns (a score-only result has no op counts),
+// computed cells and wavefront steps, and with `cycles` the device-clock breakdown
+static void count_pair(aw_batch* b, const AwPairOut& o, bool cycles) {
+    if (!(b->flags & AW_FLAG_SCORE_ONLY)) {
+        b->stats[3] += o.nruns;
+        b->stats[4] += std::max(o.n_m + o.n_x + o.n_d, o.n_m + o.n_x + o.n_i);
+    }
+    b->stats[6] += o.cells;
+    b->stats[7] += o.steps;
+    if (cycles)
+        for (int q = 0; q < 6; ++q) b->cyc[q] += o.cyc[q];
+}
+
 // joins the batch's launch (an event, not a device-wide sync: another batch of the same context may be running), copies the
 // results back on the context's copy stream and delivers them
 static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb block_cb, void* user) {
@@ -1361,14 +1361,12 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
     AW_CUDA_CHECK(cudaEventSynchronize(b->ev_done));
     cudaStream_t cs = c->copy_stream;
     int rc;
-    unsigned long long ctl[3] = {0, 0, 0};
-    if ((rc = b->h_out.ensure(sizeof(AwPairOut) * b->npairs + 64))) return rc;
-    unsigned long long* h_ctl = reinterpret_cast<unsigned long long*>(b->h_out.as<char>() + sizeof(AwPairOut) * b->npairs);  // pinned
-    AW_CUDA_CHECK(cudaMemcpyAsync(h_ctl, b->d_ctl.p, 24, cudaMemcpyDeviceToHost, cs));
+    if ((rc = b->h_out.ensure(sizeof(AwPairOut) * b->npairs + sizeof(BatchCtl)))) return rc;
+    BatchCtl* h_ctl = reinterpret_cast<BatchCtl*>(b->h_out.as<char>() + sizeof(AwPairOut) * b->npairs);  // pinned
+    AW_CUDA_CHECK(cudaMemcpyAsync(h_ctl, b->d_ctl.p, sizeof(BatchCtl), cudaMemcpyDeviceToHost, cs));
     AW_CUDA_CHECK(cudaMemcpyAsync(b->h_out.p, b->d_out.p, sizeof(AwPairOut) * b->npairs, cudaMemcpyDeviceToHost, cs));
     AW_CUDA_CHECK(cudaStreamSynchronize(cs));
-    memcpy(ctl, h_ctl, 24);
-    const uint64_t text_used = std::min<uint64_t>(ctl[0], b->text_cap), bytes_used = std::min<uint64_t>(ctl[1], b->bytes_cap);
+    const uint64_t text_used = std::min<uint64_t>(h_ctl->text_cursor, b->text_cap), bytes_used = std::min<uint64_t>(h_ctl->bytes_cursor, b->bytes_cap);
     if ((rc = b->h_text.ensure(text_used + 1)) || (rc = b->h_bytes.ensure(bytes_used + 1))) return rc;
     // block mode: the arena was re-laid out in pair order on the device (every line followed by '\n')
     const bool ordered = (b->flags & AW_FLAG_PAF_BLOCKS) && !(b->flags & AW_FLAG_NO_PAF);
@@ -1387,13 +1385,7 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
     if (blocks && all_first_try && text_used && block_cb(b->h_text.as<char>(), text_used, b->npairs, user) != 0) return AW_ECALLBACK;
     std::string sentinel;
     if (blocks && all_first_try && !cb) {  // nothing per pair is wanted: only the counters
-        for (uint64_t i = 0; i < b->npairs; ++i) {
-            const AwPairOut* o = &outs[i];
-            b->stats[3] += o->nruns;
-            b->stats[4] += std::max(o->n_m + o->n_x + o->n_d, o->n_m + o->n_x + o->n_i);
-            b->stats[6] += o->cells;
-            b->stats[7] += o->steps;
-        }
+        for (uint64_t i = 0; i < b->npairs; ++i) count_pair(b, outs[i], false);
         return AW_OK;
     }
     uint64_t ordered_off = 0;  // running offset of pair i's line in the ordered arena
@@ -1423,9 +1415,7 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
             r.score = o->score;
             r.query_end = c->lens[r.query_idx];
             r.target_end = c->lens[r.target_idx];
-            b->stats[6] += o->cells;
-            b->stats[7] += o->steps;
-            for (int q = 0; q < 6; ++q) b->cyc[q] += o->cyc[q];
+            count_pair(b, *o, true);
         } else if (o->status == AW_OK) {
             r.status = AW_OK;
             r.score = o->score;
@@ -1441,11 +1431,7 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
                 r.cigar_bytes = bytes + o->bytes_off;
                 r.cigar_len = o->n_m + o->n_x + o->n_i + o->n_d;
             }
-            b->stats[3] += o->nruns;
-            b->stats[4] += std::max(r.query_end, r.target_end);
-            b->stats[6] += o->cells;
-            b->stats[7] += o->steps;
-            for (int q = 0; q < 6; ++q) b->cyc[q] += o->cyc[q];
+            count_pair(b, *o, true);
             if (blocks && !all_first_try && block_cb(r.paf, r.paf_len + nl, 1, user) != 0) return AW_ECALLBACK;
         } else {
             // the reference's failure sentinel (src/alignment.rs:49-64) still becomes a PAF line
