@@ -984,6 +984,10 @@ int plan_launch(aw_ctx* c, const AwPen& pen, uint64_t npairs, uint64_t max_p, ui
     int hist_max_scores = attempt == 0 ? (nt == 32 ? 1024 : 4096) : (attempt == 1 ? 32768 : 262144);
     uint64_t runs_cap = max_p + max_t + 4;
     if (nt == 128 && !c->all_clean) nt = 256;  // the 128-thread kernels exist for the chunked 2-bit path only
+    // the warp-parallel leaves split the second half of the run buffer into nt / 32 parts, so a leaf gets 1 / (nt / 32) of
+    // the pair's runs: a divergent pair whose leaf needs more fails its first try, and the retry rungs give every part room
+    // for the whole pair
+    if (attempt > 0 && !use_cluster) runs_cap *= nt / 32;
     const bool ws16 = fits16 && nt >= 64;
     const uint64_t epi = ws16 ? 2 : 1;  // elements per int
     // + the all-NULL row and the compact I/D rings of the int16 path (aw_wfa.cuh: null_base, cmp_base)

@@ -95,8 +95,7 @@ def test_flag_and_scope_exported():
 def test_sweep_three_kernels(oracle, group):
     """2,000 seeded pairs per penalty set through the one-warp kernel (threads_per_cta 0: pairs up to 1 kb) and the chunked
     int16 kernels with 128 and 256 threads: scores equal the oracle's, everything else equals the full path with the default
-    kernel choice (a forced CTA size can leave the full path's deeper recursion short of workspace, which score-only never
-    reaches)"""
+    kernel choice (test_chunked_kernels.py holds the full path on the forced CTA sizes to the oracle)"""
     pen = PENALTY_SETS[group]
     ids, seqs, pairs = _sweep_group(9100 + group, npairs=2000)
     exp = oracle.run_pairs(ids, seqs, pairs, oracle.params(**pen), use_mash=True, threads=CORES)["scores"]
