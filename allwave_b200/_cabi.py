@@ -15,6 +15,7 @@ AW_OK = 0
 AW_EINVAL, AW_ENODEVICE, AW_ECUDA, AW_ENOMEM, AW_EUNSUPPORTED, AW_EWORKSPACE, AW_ECALLBACK, AW_EALIGN = -1, -2, -3, -4, -5, -6, -7, -8
 AW_ORIENT_MASH, AW_ORIENT_WFA, AW_ORIENT_FORWARD = 0, 1, 2
 AW_FLAG_CIGAR_BYTES, AW_FLAG_ORDERED, AW_FLAG_NO_PAF, AW_FLAG_PAF_BLOCKS, AW_FLAG_SCORE_ONLY = 1, 2, 4, 8, 16
+AW_FLAG_CS, AW_FLAG_CS_LONG = 32, 64
 AW_MEMORY_HIGH, AW_MEMORY_MEDIUM, AW_MEMORY_LOW, AW_MEMORY_ULTRALOW = 0, 1, 2, 3
 AW_SCOPE_SCORE, AW_SCOPE_ALIGNMENT = 0, 1
 
@@ -64,6 +65,8 @@ class AwResult(C.Structure):
         ("cg_len", C.c_uint64),
         ("paf", C.POINTER(C.c_char)),
         ("paf_len", C.c_uint64),
+        ("cs", C.POINTER(C.c_char)),
+        ("cs_len", C.c_uint64),
     ]
 
 
@@ -177,6 +180,7 @@ def result_to_dict(r, want_bytes=True):
         "num_matches": r.num_matches, "alignment_length": r.alignment_length,
         "cg": C.string_at(r.cg, r.cg_len).decode() if r.cg_len else "",
         "paf": C.string_at(r.paf, r.paf_len).decode() if r.paf_len else "",
+        "cs": C.string_at(r.cs, r.cs_len).decode() if r.cs_len else "",
     }
     if want_bytes and r.cigar_len and r.cigar_bytes:
         d["cigar_bytes"] = C.string_at(r.cigar_bytes, r.cigar_len)

@@ -16,6 +16,7 @@
 #include "aw_common.cuh"
 #include "aw_sketch.cuh"
 #include "aw_wfa.cuh"
+#include "aw_cs.cuh"
 
 static thread_local char g_err[512] = "";
 void aw_set_error(const char* fmt, ...) {
@@ -221,25 +222,29 @@ struct BatchCtl {
     unsigned long long next_pair;                  // main pass: next entry of the work list
     unsigned long long orient_next_pair[2];        // orientation passes: next entry of the work list, per strand
     unsigned long long orient_text_cursor, orient_bytes_cursor;
+    unsigned long long tag_cursor;                 // AW_FLAG_CS: bytes used in the tag arena
 };
 
 struct aw_batch {
     AwPen pen;
     int orient = AW_ORIENT_MASH;
-    uint32_t flags = 0;
+    uint32_t flags = 0;   // as the caller gave them (AW_FLAG_CS_LONG adds AW_FLAG_CS)
+    uint32_t kflags = 0;  // what the alignment passes are told: AW_FLAG_CS needs the CIGAR op bytes, and no kernel reads the CS bits
     uint64_t npairs = 0;
     std::vector<aw_pair> h_pairs;
     DevBuf d_pairs, d_isrev, d_order, d_out, d_text, d_bytes, d_ctl;
-    DevBuf d_text2, d_off;              // AW_FLAG_PAF_BLOCKS: the text arena again in pair order, and the per-pair offsets (n+1)
+    DevBuf d_text2, d_off;              // AW_FLAG_PAF_BLOCKS / AW_FLAG_CS: the text arena again in pair order, and the per-pair offsets (n+1)
+    DevBuf d_tags, d_cs_out;            // AW_FLAG_CS: the tag arena and where each pair's tag lies in it
     DevBuf d_out_f, d_out_r, d_strand;  // --wfa-orientation passes: per-strand results and a constant 0.. / 1.. strand array
     AwPen pen_orient;
-    uint64_t text_cap = 0, bytes_cap = 0;
+    uint64_t text_cap = 0, bytes_cap = 0, text2_cap = 0, tag_cap = 0;
     bool has_order = false;
     uint64_t max_p = 0, max_t = 0;
     // host copies
     PinBuf h_out, h_text, h_bytes;
     // retry pass results
     std::vector<AwPairOut> r_out;
+    std::vector<uint64_t> r_cs_len;  // AW_FLAG_CS: tag length of each r_out entry (its line in r_text carries the cs column)
     std::vector<uint32_t> r_idx;
     std::vector<char> r_text;
     std::vector<uint8_t> r_bytes;
@@ -720,14 +725,22 @@ extern "C" void aw_batch_destroy(aw_ctx* c, aw_batch* b) {
     delete b;
 }
 
-// score-only results carry no CIGAR and no PAF text
+// score-only results carry no CIGAR and no PAF text, and the cs:Z: tag is a PAF column
 static int check_flags(uint32_t flags) {
     if ((flags & AW_FLAG_SCORE_ONLY) && (flags & (AW_FLAG_CIGAR_BYTES | AW_FLAG_PAF_BLOCKS))) {
         aw_set_error("AW_FLAG_SCORE_ONLY cannot be combined with AW_FLAG_CIGAR_BYTES or AW_FLAG_PAF_BLOCKS");
         return AW_EINVAL;
     }
+    if ((flags & (AW_FLAG_CS | AW_FLAG_CS_LONG)) && (flags & (AW_FLAG_NO_PAF | AW_FLAG_SCORE_ONLY))) {
+        aw_set_error("AW_FLAG_CS / AW_FLAG_CS_LONG cannot be combined with AW_FLAG_NO_PAF or AW_FLAG_SCORE_ONLY");
+        return AW_EINVAL;
+    }
     return AW_OK;
 }
+
+// the pair-order re-layout of the text arena: whole blocks for the block callback, and one contiguous line per pair with its
+// cs column
+static bool ordered_text(uint32_t flags) { return ((flags & AW_FLAG_PAF_BLOCKS) && !(flags & AW_FLAG_NO_PAF)) || (flags & AW_FLAG_CS); }
 
 // (re)initialises a batch object for a new pair list; device / pinned buffers of an earlier use are kept (grow-only)
 static int batch_init(aw_ctx* c, aw_batch* b, const aw_params* params, int orientation_mode, const aw_pair* pairs, uint64_t npairs, uint32_t flags) {
@@ -736,7 +749,9 @@ static int batch_init(aw_ctx* c, aw_batch* b, const aw_params* params, int orien
     if (orientation_mode == AW_ORIENT_WFA && (rc = pen_from_params(&c->orient_params, &b->pen_orient))) return rc;
     b->orient = orientation_mode;
     if (flags & AW_FLAG_SCORE_ONLY) flags |= AW_FLAG_NO_PAF;
+    if (flags & AW_FLAG_CS_LONG) flags |= AW_FLAG_CS;
     b->flags = flags;
+    b->kflags = (flags & ~(AW_FLAG_CS | AW_FLAG_CS_LONG)) | ((flags & AW_FLAG_CS) ? AW_FLAG_CIGAR_BYTES : 0u);
     b->npairs = npairs;
     b->launched = false;
     b->has_order = false;
@@ -760,14 +775,17 @@ static int batch_init(aw_ctx* c, aw_batch* b, const aw_params* params, int orien
     b->text_cap = (flags & AW_FLAG_SCORE_ONLY) ? 16
                   : (flags & AW_FLAG_NO_PAF)    ? sum_len / 2 + 64 * npairs + 1024
                                                 : sum_len + (257 + 2 * idlen_max) * npairs + 1024;
-    b->bytes_cap = (flags & AW_FLAG_CIGAR_BYTES) ? sum_len + 16 : 16;
+    b->bytes_cap = (b->kflags & AW_FLAG_CIGAR_BYTES) ? sum_len + 16 : 16;
+    b->tag_cap = (flags & AW_FLAG_CS) ? 2 * sum_len + 16 : 0;                   // a tag is at most 2 * (qlen + tlen) bytes (aw_cs.cuh)
+    b->text2_cap = b->text_cap + ((flags & AW_FLAG_CS) ? 6 * npairs + b->tag_cap : 0);  // + "\tcs:Z:" and the tag per line
     const size_t np1 = (size_t)std::max<uint64_t>(1, npairs);
     if ((rc = b->d_pairs.ensure(sizeof(aw_pair) * np1)) || (rc = b->d_isrev.ensure(np1)) || (rc = b->d_out.ensure(sizeof(AwPairOut) * np1)) ||
         (rc = b->d_text.ensure(b->text_cap)) || (rc = b->d_bytes.ensure(b->bytes_cap)) || (rc = b->d_ctl.ensure(sizeof(BatchCtl))) ||
         (orientation_mode == AW_ORIENT_WFA &&
          ((rc = b->d_out_f.ensure(sizeof(AwPairOut) * np1)) || (rc = b->d_out_r.ensure(sizeof(AwPairOut) * np1)) || (rc = b->d_strand.ensure(2 * np1)))))
         return rc;
-    if ((flags & AW_FLAG_PAF_BLOCKS) && !(flags & AW_FLAG_NO_PAF) && ((rc = b->d_text2.ensure(b->text_cap)) || (rc = b->d_off.ensure(8 * (np1 + 1))))) return rc;
+    if (ordered_text(flags) && ((rc = b->d_text2.ensure(b->text2_cap)) || (rc = b->d_off.ensure(8 * (np1 + 1))))) return rc;
+    if ((flags & AW_FLAG_CS) && ((rc = b->d_tags.ensure(b->tag_cap)) || (rc = b->d_cs_out.ensure(sizeof(AwCsOut) * np1)))) return rc;
     // uploads go through their own stream, so that a batch can be prepared while the previous one is still running
     cudaStream_t us = c->up_stream;
     cudaError_t e = cudaMemcpyAsync(b->d_pairs.p, pairs, sizeof(aw_pair) * npairs, cudaMemcpyHostToDevice, us);
@@ -1118,6 +1136,21 @@ cudaError_t launch_orientation(aw_ctx* c, aw_batch* b, const LaunchCfg& cfo, con
     return cudaSuccess;
 }
 
+// the cs:Z: tags of the pairs order[0 .. npairs) (0 .. npairs without an order) of an alignment pass: results `out`, CIGAR op
+// bytes `ops`; tags into the arena `tags` at the cursor, their places into cs_out
+cudaError_t launch_cs(aw_ctx* c, aw_batch* b, const AwPairOut* out, const uint32_t* order, uint64_t npairs, const uint8_t* ops, char* tags,
+                      unsigned long long* tag_cursor, AwCsOut* cs_out, cudaStream_t st) {
+    const unsigned grid = (unsigned)std::min<uint64_t>(npairs, 1u << 20);
+    const int long_form = (b->flags & AW_FLAG_CS_LONG) ? 1 : 0;
+    if (b->max_p + b->max_t <= awk::CS_SHORT_LEN)
+        awk::aw_cs_kernel<awk::CS_NT_SHORT><<<grid, awk::CS_NT_SHORT, 0, st>>>(out, order, (uint32_t)npairs, b->d_pairs.as<aw_pair>(), c->d_slots.as<AwSlot>(),
+                                                                             c->d_ascii.as<uint8_t>(), ops, long_form, tags, tag_cursor, cs_out);
+    else
+        awk::aw_cs_kernel<awk::CS_NT><<<grid, awk::CS_NT, 0, st>>>(out, order, (uint32_t)npairs, b->d_pairs.as<aw_pair>(), c->d_slots.as<AwSlot>(),
+                                                                 c->d_ascii.as<uint8_t>(), ops, long_form, tags, tag_cursor, cs_out);
+    return cudaGetLastError();
+}
+
 }  // namespace
 
 extern "C" int aw_batch_launch(aw_ctx* c, aw_batch* b, void* stream) {
@@ -1128,6 +1161,7 @@ extern "C" int aw_batch_launch(aw_ctx* c, aw_batch* b, void* stream) {
     memset(b->stats, 0, sizeof(b->stats));
     memset(b->cyc, 0, sizeof(b->cyc));
     b->r_out.clear();
+    b->r_cs_len.clear();
     b->r_idx.clear();
     b->r_text.clear();
     b->r_bytes.clear();
@@ -1166,17 +1200,25 @@ extern "C" int aw_batch_launch(aw_ctx* c, aw_batch* b, void* stream) {
         AW_CUDA_CHECK(cudaEventCreateWithFlags(&b->ev_done, cudaEventDisableTiming));
     }
     AW_CUDA_CHECK(cudaEventRecord(b->ev0, st));
-    cudaError_t e = launch_pass(c, b, b->pen, cfg, b->flags, b->d_isrev.as<uint8_t>(), order, b->npairs, b->d_out.as<AwPairOut>(), b->d_text.as<char>(),
+    cudaError_t e = launch_pass(c, b, b->pen, cfg, b->kflags, b->d_isrev.as<uint8_t>(), order, b->npairs, b->d_out.as<AwPairOut>(), b->d_text.as<char>(),
                                 b->text_cap, b->d_bytes.as<uint8_t>(), b->bytes_cap, &ctl->text_cursor, &ctl->bytes_cursor, &ctl->next_pair, st);
     if (e != cudaSuccess) {
         aw_set_error("align kernel launch (nt=%d grid=%d): %s", cfg.nt, cfg.grid, cudaGetErrorString(e));
         return AW_ECUDA;
     }
     AW_CUDA_CHECK(cudaEventRecord(b->ev1, st));
-    if ((b->flags & AW_FLAG_PAF_BLOCKS) && !(b->flags & AW_FLAG_NO_PAF)) {
-        awk::aw_text_scan_kernel<<<1, 1024, 0, st>>>(b->d_out.as<AwPairOut>(), (uint32_t)b->npairs, b->d_off.as<unsigned long long>());
+    const bool cs = (b->flags & AW_FLAG_CS) != 0;
+    if (cs) {
+        AW_CUDA_CHECK(launch_cs(c, b, b->d_out.as<AwPairOut>(), nullptr, b->npairs, b->d_bytes.as<uint8_t>(), b->d_tags.as<char>(), &ctl->tag_cursor,
+                                b->d_cs_out.as<AwCsOut>(), st));
+        ++b->stats[0];
+    }
+    if (ordered_text(b->flags)) {
+        const AwCsOut* cs_out = cs ? b->d_cs_out.as<AwCsOut>() : nullptr;
+        const unsigned nl = (b->flags & AW_FLAG_PAF_BLOCKS) ? 1u : 0u;
+        awk::aw_text_scan_kernel<<<1, 1024, 0, st>>>(b->d_out.as<AwPairOut>(), cs_out, nl, (uint32_t)b->npairs, b->d_off.as<unsigned long long>());
         awk::aw_text_gather_kernel<<<c->sm_count * 8, 256, 0, st>>>(b->d_out.as<AwPairOut>(), b->d_off.as<unsigned long long>(), (uint32_t)b->npairs,
-                                                                  b->d_text.as<char>(), b->d_text2.as<char>());
+                                                                  b->d_text.as<char>(), cs_out, b->d_tags.as<char>(), nl, b->d_text2.as<char>());
         AW_CUDA_CHECK(cudaGetLastError());
         b->stats[0] += 2;
     }
@@ -1284,6 +1326,7 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
         if (rc) return rc;
     }
     const unsigned nl = (b->flags & AW_FLAG_PAF_BLOCKS) ? 1u : 0u;
+    const bool cs = (b->flags & AW_FLAG_CS) != 0;
     for (int attempt = 1; attempt <= 3 && !failed.empty(); ++attempt) {
         const bool give_up = attempt > c->max_retry;  // ladder disabled or exhausted: report the pairs as failed
         if (give_up) {
@@ -1292,6 +1335,7 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
                 o.status = AW_EALIGN;
                 b->r_idx.push_back(i);
                 b->r_out.push_back(o);
+                b->r_cs_len.push_back(0);
             }
             failed.clear();
             break;
@@ -1303,15 +1347,22 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
             idlen_max = std::max(idlen_max, c->ids[b->h_pairs[i].query_idx].size() + c->ids[b->h_pairs[i].target_idx].size());
         }
         const uint64_t text_cap = 12 * sum_len + (256 + idlen_max) * failed.size() + 1024;
-        const uint64_t bytes_cap = (b->flags & AW_FLAG_CIGAR_BYTES) ? sum_len + 16 : 16;
-        DevBuf d_out, d_text, d_bytes;
+        const uint64_t bytes_cap = (b->kflags & AW_FLAG_CIGAR_BYTES) ? sum_len + 16 : 16;
+        const uint64_t tag_cap = cs ? 2 * sum_len + 16 : 0;
+        DevBuf d_out, d_text, d_bytes, d_tags, d_cs_out;
         auto launch = [&](const LaunchCfg& cfg, const uint32_t* order, BatchCtl* ctl, cudaStream_t kst) -> int {
             int rc;
             if ((rc = d_out.ensure(sizeof(AwPairOut) * b->npairs)) || (rc = d_text.ensure(text_cap)) || (rc = d_bytes.ensure(bytes_cap))) return rc;
-            const cudaError_t e = launch_pass(c, b, b->pen, cfg, b->flags, b->d_isrev.as<uint8_t>(), order, failed.size(), d_out.as<AwPairOut>(),
-                                              d_text.as<char>(), text_cap, d_bytes.as<uint8_t>(), bytes_cap, &ctl->text_cursor, &ctl->bytes_cursor,
-                                              &ctl->next_pair, kst);
+            if (cs && ((rc = d_tags.ensure(tag_cap)) || (rc = d_cs_out.ensure(sizeof(AwCsOut) * b->npairs)))) return rc;
+            cudaError_t e = launch_pass(c, b, b->pen, cfg, b->kflags, b->d_isrev.as<uint8_t>(), order, failed.size(), d_out.as<AwPairOut>(),
+                                        d_text.as<char>(), text_cap, d_bytes.as<uint8_t>(), bytes_cap, &ctl->text_cursor, &ctl->bytes_cursor,
+                                        &ctl->next_pair, kst);
             ++b->stats[0];
+            if (e == cudaSuccess && cs) {
+                e = launch_cs(c, b, d_out.as<AwPairOut>(), order, failed.size(), d_bytes.as<uint8_t>(), d_tags.as<char>(), &ctl->tag_cursor,
+                              d_cs_out.as<AwCsOut>(), kst);
+                ++b->stats[0];
+            }
             if (e != cudaSuccess) aw_set_error("retry launch: %s", cudaGetErrorString(e));
             return e == cudaSuccess ? AW_OK : AW_ECUDA;
         };
@@ -1319,9 +1370,13 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
         BatchCtl ctl;
         if (int rc = retry_rung(c, b, b->pen, failed, attempt, "retry launch", launch, {{&d_out, &outs}}, &ctl)) return rc;
         std::vector<char> text(std::min<uint64_t>(ctl.text_cursor, text_cap));
-        std::vector<uint8_t> bytes(std::min<uint64_t>(ctl.bytes_cursor, bytes_cap));
+        std::vector<uint8_t> bytes((b->flags & AW_FLAG_CIGAR_BYTES) ? std::min<uint64_t>(ctl.bytes_cursor, bytes_cap) : 0);
+        std::vector<char> tags(cs ? std::min<uint64_t>(ctl.tag_cursor, tag_cap) : 0);
+        std::vector<AwCsOut> cs_out(cs ? b->npairs : 0);
         if (!text.empty()) AW_CUDA_CHECK(cudaMemcpy(text.data(), d_text.p, text.size(), cudaMemcpyDeviceToHost));
         if (!bytes.empty()) AW_CUDA_CHECK(cudaMemcpy(bytes.data(), d_bytes.p, bytes.size(), cudaMemcpyDeviceToHost));
+        if (!tags.empty()) AW_CUDA_CHECK(cudaMemcpy(tags.data(), d_tags.p, tags.size(), cudaMemcpyDeviceToHost));
+        if (cs) AW_CUDA_CHECK(cudaMemcpy(cs_out.data(), d_cs_out.p, sizeof(AwCsOut) * b->npairs, cudaMemcpyDeviceToHost));
         std::vector<uint32_t> still;
         for (uint32_t i : failed) {
             AwPairOut o = outs[i];
@@ -1329,9 +1384,18 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
                 still.push_back(i);
                 continue;
             }
+            uint64_t cs_len = 0;
             if (o.status == AW_OK) {
                 const uint64_t toff = b->r_text.size(), boff = b->r_bytes.size();
-                b->r_text.insert(b->r_text.end(), text.begin() + o.paf_off, text.begin() + o.paf_off + o.paf_len + (o.paf_len ? nl : 0));
+                // the line, then the cs column, then the newline of block mode
+                b->r_text.insert(b->r_text.end(), text.begin() + o.paf_off, text.begin() + o.paf_off + o.paf_len);
+                if (cs) {
+                    static const char col[] = "\tcs:Z:";
+                    cs_len = cs_out[i].len;
+                    b->r_text.insert(b->r_text.end(), col, col + 6);
+                    b->r_text.insert(b->r_text.end(), tags.begin() + cs_out[i].off, tags.begin() + cs_out[i].off + cs_len);
+                }
+                if (o.paf_len && nl) b->r_text.push_back('\n');
                 const uint64_t nb = (b->flags & AW_FLAG_CIGAR_BYTES) ? o.n_m + o.n_x + o.n_i + o.n_d : 0;
                 if (nb) b->r_bytes.insert(b->r_bytes.end(), bytes.begin() + o.bytes_off, bytes.begin() + o.bytes_off + nb);
                 o.paf_off = toff;
@@ -1339,6 +1403,7 @@ static int retry_failed(aw_ctx* c, aw_batch* b, const AwPairOut* h_out) {
             }
             b->r_idx.push_back(i);
             b->r_out.push_back(o);
+            b->r_cs_len.push_back(cs_len);
         }
         failed.swap(still);
     }
@@ -1364,16 +1429,26 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
     if (b->npairs == 0) return AW_OK;
     AW_CUDA_CHECK(cudaEventSynchronize(b->ev_done));
     cudaStream_t cs = c->copy_stream;
+    const bool with_cs = (b->flags & AW_FLAG_CS) != 0;
     int rc;
-    if ((rc = b->h_out.ensure(sizeof(AwPairOut) * b->npairs + sizeof(BatchCtl)))) return rc;
-    BatchCtl* h_ctl = reinterpret_cast<BatchCtl*>(b->h_out.as<char>() + sizeof(AwPairOut) * b->npairs);  // pinned
+    // pinned: the results, the control block, and with AW_FLAG_CS the ordered arena's size and every pair's tag place
+    if ((rc = b->h_out.ensure(sizeof(AwPairOut) * b->npairs + sizeof(BatchCtl) + 8 + (with_cs ? sizeof(AwCsOut) * b->npairs : 0)))) return rc;
+    BatchCtl* h_ctl = reinterpret_cast<BatchCtl*>(b->h_out.as<char>() + sizeof(AwPairOut) * b->npairs);
+    unsigned long long* h_ordered_len = reinterpret_cast<unsigned long long*>(h_ctl + 1);
+    const AwCsOut* h_cs = reinterpret_cast<const AwCsOut*>(h_ordered_len + 1);
     AW_CUDA_CHECK(cudaMemcpyAsync(h_ctl, b->d_ctl.p, sizeof(BatchCtl), cudaMemcpyDeviceToHost, cs));
     AW_CUDA_CHECK(cudaMemcpyAsync(b->h_out.p, b->d_out.p, sizeof(AwPairOut) * b->npairs, cudaMemcpyDeviceToHost, cs));
+    if (with_cs) {
+        AW_CUDA_CHECK(cudaMemcpyAsync(h_ordered_len, b->d_off.as<unsigned long long>() + b->npairs, 8, cudaMemcpyDeviceToHost, cs));
+        AW_CUDA_CHECK(cudaMemcpyAsync((void*)h_cs, b->d_cs_out.p, sizeof(AwCsOut) * b->npairs, cudaMemcpyDeviceToHost, cs));
+    }
     AW_CUDA_CHECK(cudaStreamSynchronize(cs));
-    const uint64_t text_used = std::min<uint64_t>(h_ctl->text_cursor, b->text_cap), bytes_used = std::min<uint64_t>(h_ctl->bytes_cursor, b->bytes_cap);
+    const uint64_t text_used = with_cs ? std::min<uint64_t>(*h_ordered_len, b->text2_cap) : std::min<uint64_t>(h_ctl->text_cursor, b->text_cap);
+    const uint64_t bytes_used = std::min<uint64_t>(h_ctl->bytes_cursor, b->bytes_cap);
     if ((rc = b->h_text.ensure(text_used + 1)) || (rc = b->h_bytes.ensure(bytes_used + 1))) return rc;
-    // block mode: the arena was re-laid out in pair order on the device (every line followed by '\n')
-    const bool ordered = (b->flags & AW_FLAG_PAF_BLOCKS) && !(b->flags & AW_FLAG_NO_PAF);
+    // block mode and AW_FLAG_CS: the arena was re-laid out in pair order on the device (every line followed by '\n' in block
+    // mode, and by its cs column with AW_FLAG_CS)
+    const bool ordered = ordered_text(b->flags);
     if (text_used) AW_CUDA_CHECK(cudaMemcpyAsync(b->h_text.p, ordered ? b->d_text2.p : b->d_text.p, text_used, cudaMemcpyDeviceToHost, cs));
     if (bytes_used && (b->flags & AW_FLAG_CIGAR_BYTES)) AW_CUDA_CHECK(cudaMemcpyAsync(b->h_bytes.p, b->d_bytes.p, bytes_used, cudaMemcpyDeviceToHost, cs));
     AW_CUDA_CHECK(cudaStreamSynchronize(cs));
@@ -1393,20 +1468,23 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
         return AW_OK;
     }
     uint64_t ordered_off = 0;  // running offset of pair i's line in the ordered arena
+    static const char cs_col[] = "\tcs:Z:";
     for (uint64_t i = 0; i < b->npairs; ++i) {
         const AwPairOut* o = &outs[i];
         const char* text = b->h_text.as<char>();
         const uint8_t* bytes = b->h_bytes.as<uint8_t>();
         uint64_t paf_off = o->paf_off;
+        uint64_t cs_len = with_cs ? h_cs[i].len : 0;
         if (ordered) {
             paf_off = ordered_off;
-            if (o->status == AW_OK && o->paf_len) ordered_off += o->paf_len + 1ull;
+            if (o->status == AW_OK && o->paf_len) ordered_off += o->paf_len + nl + (with_cs ? 6 + cs_len : 0);
         }
         if (!retry_of.empty() && retry_of[i] >= 0) {
             o = &b->r_out[retry_of[i]];
             text = b->r_text.data();
             bytes = b->r_bytes.data();
             paf_off = o->paf_off;
+            cs_len = with_cs ? b->r_cs_len[retry_of[i]] : 0;
         }
         aw_result r;
         memset(&r, 0, sizeof(r));
@@ -1428,9 +1506,13 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
             r.num_matches = o->n_m;
             r.alignment_length = o->n_m + o->n_x;
             r.paf = (b->flags & AW_FLAG_NO_PAF) ? nullptr : text + paf_off;
-            r.paf_len = (b->flags & AW_FLAG_NO_PAF) ? 0 : o->paf_len;
+            r.paf_len = (b->flags & AW_FLAG_NO_PAF) ? 0 : o->paf_len + (with_cs ? 6 + cs_len : 0);
             r.cg = text + paf_off + o->cg_off;
             r.cg_len = o->paf_len - o->cg_off;
+            if (with_cs) {
+                r.cs = text + paf_off + o->paf_len + 6;
+                r.cs_len = cs_len;
+            }
             if (b->flags & AW_FLAG_CIGAR_BYTES) {
                 r.cigar_bytes = bytes + o->bytes_off;
                 r.cigar_len = o->n_m + o->n_x + o->n_i + o->n_d;
@@ -1450,10 +1532,13 @@ static int fetch_impl(aw_ctx* c, aw_batch* b, aw_result_cb cb, aw_paf_block_cb b
                 sentinel += c->ids[r.target_idx];
                 snprintf(buf, sizeof(buf), "\t%llu\t0\t0\t0\t0\t60\tgi:f:0.000000\tcg:Z:", (unsigned long long)c->lens[r.target_idx]);
                 sentinel += buf;
+                const size_t cg_end = sentinel.size();
+                if (with_cs) sentinel += cs_col;
                 if (nl) sentinel += '\n';
                 r.paf = sentinel.data();
                 r.paf_len = sentinel.size() - nl;
-                r.cg = r.paf + r.paf_len;
+                r.cg = r.paf + cg_end;
+                if (with_cs) r.cs = r.paf + r.paf_len;
                 if (blocks && block_cb(r.paf, r.paf_len + nl, 1, user) != 0) return AW_ECALLBACK;
             }
         }

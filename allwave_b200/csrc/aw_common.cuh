@@ -59,6 +59,11 @@ struct AwPairOut {
     unsigned long long cyc[6];
 };
 
+// where the cs:Z: value of a pair (AW_FLAG_CS) lies in the tag arena
+struct AwCsOut {
+    unsigned long long off, len;
+};
+
 #define AW_CUDA_CHECK(call)                                                         \
     do {                                                                            \
         cudaError_t _e = (call);                                                    \

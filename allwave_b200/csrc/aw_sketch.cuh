@@ -307,16 +307,22 @@ __global__ void aw_wfa_orient_pick_kernel(const AwPairOut* __restrict__ fwd, con
     }
 }
 
-// ---- ordered PAF text (AW_FLAG_PAF_BLOCKS): the alignment kernel appends lines to the text arena in completion order; these
-// two kernels lay them out again in PAIR order (the order the reference's writer sees with one worker thread,
-// src/main.rs:347-374), so a whole batch leaves the GPU as one ready-to-write block of newline-terminated lines.
-// off[i] = byte offset of pair i's line in the ordered arena, off[n] = total; one block, exclusive scan of (paf_len + 1)
-__global__ void aw_text_scan_kernel(const AwPairOut* __restrict__ out, uint32_t n, unsigned long long* __restrict__ off) {
+// ---- ordered PAF text (AW_FLAG_PAF_BLOCKS, AW_FLAG_CS): the alignment kernel appends lines to the text arena in completion
+// order; these two kernels lay them out again in PAIR order (the order the reference's writer sees with one worker thread,
+// src/main.rs:347-374), so a whole batch leaves the GPU as one ready-to-write block of lines.  A line is followed by '\n'
+// when nl is 1, and with cs (AW_FLAG_CS) it gains the column "\tcs:Z:" + the pair's tag before that.
+__device__ __forceinline__ unsigned long long ordered_line_len(const AwPairOut& o, const AwCsOut* cs, uint32_t i, unsigned nl) {
+    if (o.status != AW_OK || o.paf_len == 0) return 0;
+    return o.paf_len + nl + (cs ? 6 + cs[i].len : 0);
+}
+// off[i] = byte offset of pair i's line in the ordered arena, off[n] = total; one block, exclusive scan of the line lengths
+__global__ void aw_text_scan_kernel(const AwPairOut* __restrict__ out, const AwCsOut* __restrict__ cs, unsigned nl, uint32_t n,
+                                    unsigned long long* __restrict__ off) {
     __shared__ unsigned long long part[1024];
     const uint32_t per = (n + blockDim.x - 1) / blockDim.x;
     const uint32_t b = min(n, threadIdx.x * per), e = min(n, b + per);
     unsigned long long sum = 0;
-    for (uint32_t i = b; i < e; ++i) sum += (out[i].status == AW_OK && out[i].paf_len) ? out[i].paf_len + 1ull : 0ull;
+    for (uint32_t i = b; i < e; ++i) sum += ordered_line_len(out[i], cs, i, nl);
     part[threadIdx.x] = sum;
     __syncthreads();
     for (unsigned d = 1; d < blockDim.x; d <<= 1) {
@@ -328,13 +334,13 @@ __global__ void aw_text_scan_kernel(const AwPairOut* __restrict__ out, uint32_t 
     unsigned long long run = part[threadIdx.x] - sum;
     for (uint32_t i = b; i < e; ++i) {
         off[i] = run;
-        run += (out[i].status == AW_OK && out[i].paf_len) ? out[i].paf_len + 1ull : 0ull;
+        run += ordered_line_len(out[i], cs, i, nl);
     }
     if (threadIdx.x == blockDim.x - 1) off[n] = part[threadIdx.x];
 }
-// one warp per pair: copy line + '\n' from the completion-order arena to its slot of the ordered arena
+// one warp per pair: copy the line (+ the cs column from the tag arena) (+ '\n') to its slot of the ordered arena
 __global__ void aw_text_gather_kernel(const AwPairOut* __restrict__ out, const unsigned long long* __restrict__ off, uint32_t n, const char* __restrict__ src,
-                                      char* __restrict__ dst) {
+                                      const AwCsOut* __restrict__ cs, const char* __restrict__ tags, unsigned nl, char* __restrict__ dst) {
     const uint64_t warp = (blockIdx.x * (uint64_t)blockDim.x + threadIdx.x) >> 5;
     const uint64_t nwarps = ((uint64_t)gridDim.x * blockDim.x) >> 5;
     const unsigned lane = threadIdx.x & 31;
@@ -342,8 +348,18 @@ __global__ void aw_text_gather_kernel(const AwPairOut* __restrict__ out, const u
         if (out[p].status != AW_OK || out[p].paf_len == 0) continue;
         const char* s = src + out[p].paf_off;
         char* d = dst + off[p];
-        const unsigned len = out[p].paf_len + 1;
+        const unsigned len = out[p].paf_len;
         for (unsigned i = lane; i < len; i += 32) d[i] = s[i];
+        d += len;
+        if (cs) {
+            const char col[6] = {'\t', 'c', 's', ':', 'Z', ':'};
+            if (lane < 6) d[lane] = col[lane];
+            const char* t = tags + cs[p].off;
+            const unsigned long long tl = cs[p].len;
+            for (unsigned long long i = lane; i < tl; i += 32) d[6 + i] = t[i];
+            d += 6 + tl;
+        }
+        if (nl && lane == 0) *d = '\n';
     }
 }
 

@@ -445,11 +445,12 @@ class AllPairIterator {
     void for_each_with_callback_multi(const std::vector<Context*>& others, const Callback& cb, uint32_t flags = 0) { for_each_with_callback(cb, flags, others); }
     // PAF writer paths of the CLI (src/main.rs:347-374).  Blocks: newline-terminated PAF lines exactly as they leave the
     // GPU (within a block the lines are in pair order; with one GPU the blocks are too), no per-pair host work at all.
+    // `flags` adds aw_align_stream flags, e.g. AW_FLAG_CS for the cs:Z: column.
     using BlockCallback = std::function<void(const char* text, size_t len, size_t n_lines)>;
-    void for_each_paf_block(const BlockCallback& cb, const std::vector<Context*>& others = {}) {
+    void for_each_paf_block(const BlockCallback& cb, const std::vector<Context*>& others = {}, uint32_t flags = 0) {
         Delivery d;
         d.block = &cb;
-        drive(d, AW_FLAG_PAF_BLOCKS, others);
+        drive(d, AW_FLAG_PAF_BLOCKS | flags, others);
     }
     // one call per line (without the newline)
     using PafCallback = std::function<void(const char*, size_t)>;

@@ -1,6 +1,6 @@
 // allwave_cli.cpp -- minimal driver with allwave's CLI surface for the alignment path
 // (src/main.rs:32-80): -i FASTA[.gz] [-o PAF] [-s scores | -x ANI preset] [-p strategy] [-t N] [-k prefixes | -e prefixes]
-// [--mash-matrix] [--wfa-orientation] [--no-progress] [--gpu D] [--gpus N].  FASTA parsing and the PAF writer thread stay on
+// [--mash-matrix] [--wfa-orientation] [--cs[=short|long]] [--no-progress] [--gpu D] [--gpus N].  FASTA parsing and the PAF writer thread stay on
 // the host; everything between the pair list and the ready-to-write PAF text runs on the GPU through liballwave_cuda.so.
 #include <chrono>
 #include <cstdio>
@@ -63,6 +63,7 @@ int main(int argc, char** argv) {
     std::string input, output, scores = "0,5,8,2,24,1", spars = "giant:0.99", preset, keep_prefixes, exclude_prefixes;
     bool wfa_orientation = false, progress = true, mash_matrix = false, scores_given = false;
     int device = 0, gpus = 1, threads = 1;
+    uint32_t cs_flags = 0;  // --cs: minimap2's cs:Z: column on every PAF line (short form; --cs=long: long form)
     for (int i = 1; i < argc; ++i) {
         std::string a = argv[i];
         auto need = [&](const char* name) -> std::string {
@@ -86,11 +87,17 @@ int main(int argc, char** argv) {
         else if (a == "--gpu") device = std::atoi(need("--gpu").c_str());
         else if (a == "--gpus") gpus = std::max(1, std::atoi(need("--gpus").c_str()));  // devices device .. device+gpus-1, pairs sharded by predicted cost
         else if (a == "--wfa-orientation") wfa_orientation = true;
+        else if (a == "--cs" || a == "--cs=short") cs_flags = AW_FLAG_CS;
+        else if (a == "--cs=long") cs_flags = AW_FLAG_CS | AW_FLAG_CS_LONG;
+        else if (a.rfind("--cs=", 0) == 0) {
+            std::fprintf(stderr, "error: --cs takes 'short' or 'long', not '%s'\n", a.c_str() + 5);
+            return 2;
+        }
         else if (a == "--no-progress") progress = false;
         else {
             std::fprintf(stderr,
                          "usage: allwave -i FASTA[.gz] [-o PAF] [-s scores | -x ANI] [-p none|auto|random:f|giant:p|tree:n:f:r[:k]] [-k prefixes | -e prefixes]\n"
-                         "               [--mash-matrix] [--wfa-orientation] [--no-progress] [--gpu D] [--gpus N]\n");
+                         "               [--mash-matrix] [--wfa-orientation] [--cs[=short|long]] [--no-progress] [--gpu D] [--gpus N]\n");
             return 2;
         }
     }
@@ -177,7 +184,7 @@ int main(int argc, char** argv) {
                 writer.push(text, len);
                 done += n_lines;
             },
-            others);
+            others, cs_flags);
         mark("last PAF block delivered");
         writer.close();
         if (out != stdout) std::fclose(out);

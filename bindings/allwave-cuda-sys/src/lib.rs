@@ -27,6 +27,8 @@ pub const AW_FLAG_ORDERED: u32 = 2;
 pub const AW_FLAG_NO_PAF: u32 = 4;
 pub const AW_FLAG_PAF_BLOCKS: u32 = 8;
 pub const AW_FLAG_SCORE_ONLY: u32 = 16;
+pub const AW_FLAG_CS: u32 = 32;
+pub const AW_FLAG_CS_LONG: u32 = 64;
 
 // aw_memory_mode / aw_alignment_scope / aw_alignment_span / aw_heuristic / aw_alignment_status (lib_wfa2 names)
 pub const AW_MEMORY_HIGH: c_int = 0;
@@ -87,6 +89,8 @@ pub struct aw_result {
     pub cg_len: u64,
     pub paf: *const c_char,
     pub paf_len: u64,
+    pub cs: *const c_char,
+    pub cs_len: u64,
 }
 
 #[repr(C)]

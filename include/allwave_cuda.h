@@ -84,6 +84,8 @@ typedef struct aw_result {
     uint64_t cg_len;
     const char* paf;            /* alignment_to_paf line without '\n' (not NUL-terminated)            */
     uint64_t paf_len;
+    const char* cs;             /* AW_FLAG_CS: the cs:Z: value (without "cs:Z:"), the last column of paf; NULL otherwise */
+    uint64_t cs_len;
 } aw_result;
 
 /* return non-zero to cancel the run (mirrors a callback Err, src/iterator.rs:235-251) */
@@ -106,6 +108,15 @@ typedef struct aw_aligner aw_aligner;
                                    alignment_length = 0; cigar_bytes, cg and paf are NULL with length 0.  A failed pair is
                                    AW_EALIGN with score INT32_MAX (no sentinel line).  aw_batch_stats [2..4] are 0.
                                    The biWFA recursion stops at its top level, whose breakpoint score is the optimal score. */
+#define AW_FLAG_CS 32u          /* append minimap2's cs:Z: difference string (short form) to every PAF line as its last column,
+                                   "\tcs:Z:<value>", built on the GPU from the CIGAR and both sequences; result.cs points at the
+                                   value.  It describes the target against the oriented query (reverse-complemented on '-'
+                                   lines): ":N" a run of N matches, "*tq" one mismatch column (target base, query base),
+                                   "+bases" query bases absent from the target, "-bases" target bases absent from the query;
+                                   bases of "*", "+" and "-" are lower-cased.  A failure sentinel line ends in an empty
+                                   "\tcs:Z:".  cg / cg_len still cover the cg:Z: value alone.  AW_EINVAL with AW_FLAG_NO_PAF
+                                   or AW_FLAG_SCORE_ONLY */
+#define AW_FLAG_CS_LONG 64u     /* the long form of AW_FLAG_CS (implies it): "=BASES" (upper-cased target bases) instead of ":N" */
 
 /* ---- library / device ---- */
 int aw_abi_version(void);
